@@ -2,6 +2,7 @@
 """Benchmark of the hot path: Conformer encoder forward, frames/sec at max-frames=1600 (BASELINE.json).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--precision tf32|fp32]
+                    [--dump-outputs DIR]
 
 A step = one ConformerEncoder.forward (embed + 12 layers + after_norm, eval) over one synthetic max-frames=1600
 bucket per GPU (workload S2 = 4 utterances x 400 frames, d=768, BASELINE.json configs[1]); weak scaling: every
@@ -10,6 +11,8 @@ Prints ONE JSON line (rank 0).  `--impl reference` times the reference's own CPU
 instead: the unmodified espnet modules copied into the git-ignored oracle/_ref by oracle/build_ref.py (kind
 "reference"; the copy travels to the GPU box with the snapshot), or, when that copy is absent, the CPU restatement
 oracle/conformer_oracle.py (kind "port", pinned to the reference by tests/test_oracle_golden.py).
+`--dump-outputs DIR` writes what the timed path returned in its last timed step (rank 0) as DIR/<name>.npy in float32,
+so that two builds run with the same arguments, hence the same seeded inputs, can be compared output for output.
 """
 from __future__ import annotations
 
@@ -103,6 +106,15 @@ class ClockSampler:
         busy = [v for v in sm if mx and v > 0.3 * mx] or sm
         return {"sm_mhz": statistics.median(busy) if busy else None, "sm_max_mhz": mx, "reasons": sorted(reasons),
                 "samples": len(sm)}
+
+
+def dump_outputs(directory, arrays):
+    """arrays: name -> tensor; written as directory/<name>.npy in float32."""
+    import numpy as np
+    os.makedirs(directory, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(directory, name + ".npy"), t.detach().float().cpu().numpy())
+    log(f"outputs of the last timed step written to {directory}: {', '.join(sorted(arrays))}")
 
 
 def log(msg):
@@ -201,15 +213,13 @@ def run_reference(args):
     torch.set_num_threads(threads)
     cpu = CpuEncoder(CFG)
     xs = encoder_input(lengths, CFG["d_model"], 1234)
-    t0 = time.perf_counter()
     cpu.forward(xs, lengths)                                        # warm-up (1 forward; each is a full S2 bucket)
-    warm = time.perf_counter() - t0
-    if warm * args.steps > 120:                                     # keep the arm within a few minutes
-        args.steps = max(1, int(120 / warm))
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        cpu.forward(xs, lengths)
+        out = cpu.forward(xs, lengths)
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"encoder_out": out, "masks": non_pad_mask(lengths, "cpu")})
     fps = sum(lengths) * args.steps / dt
     note = ("the reference's own espnet ConformerEncoder (oracle/_ref: unmodified copy made by oracle/build_ref.py)"
             if cpu.kind == "reference" else
@@ -537,12 +547,14 @@ def run_ours(args):
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
         for i in range(args.steps):
-            enc(dev_in[i % nbuf], mask)
+            out = enc(dev_in[i % nbuf], mask)
         e1.record()
         barrier()
         ms = e0.elapsed_time(e1)
         launches = _cabi.launch_count() - l0
         log(f"device-timed region done: {ms / args.steps:.3f} ms/step")
+        if args.dump_outputs and rank == 0:
+            dump_outputs(args.dump_outputs, {"encoder_out": out[0], "masks": out[1]})
         # ---- end to end through the public API: every step copies its inputs from pinned host memory (H2D), runs
         # ConformerEncoder.forward, and copies the features back to pinned host memory (D2H).  PipelinedEncoder
         # (auto_avsr_b200/pipeline.py) overlaps the copies of neighbouring steps with the forward on 3 streams.
@@ -626,10 +638,12 @@ def main():
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
     ap.add_argument("--no-extras", action="store_true", help="skip the extras (other shapes / precisions, sustained "
                                                                "loop, eager-PyTorch GPU comparator)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step as DIR/<name>.npy "
+                                                           "(float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
-        if args.steps > 20:
-            args.steps = 20          # ~1 s per CPU forward: keep the arm within a few minutes
         run_reference(args)
     else:
         run_ours(args)

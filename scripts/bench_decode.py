@@ -85,7 +85,7 @@ def main():
         best["device"] = (nb[0].yseq.tolist(), float(nb[0].score))
         out["device_beam_search"] = {"ms_per_utterance": dt * 1e3, "steps": steps, "ms_per_step": dt * 1e3 / max(steps, 1),
                                      "utterances_per_s": 1.0 / dt, "nbest": len(nb), "best_score": float(nb[0].score),
-                                     "precision": dec.precision or "f16",
+                                     "best_yseq": best["device"][0], "precision": dec.precision or "f16",
                                      "api": "auto_avsr_b200.beam_search.DeviceBeamSearch -> avsr_decoder_step / avsr_ctc_prefix_*"}
     except Exception as e:                                   # noqa: BLE001
         out["device_beam_search"] = {"error": f"{type(e).__name__}: {e}"}
@@ -106,7 +106,7 @@ def main():
                 dt, nb = timed(lambda: bs2(x), 2)
             best["ref_loop"] = (nb[0].yseq.tolist(), float(nb[0].score))
             out["reference_loop_dropins"] = {"ms_per_utterance": dt * 1e3, "utterances_per_s": 1.0 / dt, "nbest": len(nb),
-                                             "best_score": float(nb[0].score),
+                                             "best_score": float(nb[0].score), "best_yseq": best["ref_loop"][0],
                                              "api": "espnet BatchBeamSearch (unmodified) over the drop-in scorers"}
         except Exception as e:                               # noqa: BLE001
             out["reference_loop_dropins"] = {"error": f"{type(e).__name__}: {e}"}
@@ -121,7 +121,7 @@ def main():
                 dt, nb = timed(lambda: bs3(x), 1)
             best["ref_eager"] = (nb[0].yseq.tolist(), float(nb[0].score))
             out["reference_eager"] = {"ms_per_utterance": dt * 1e3, "utterances_per_s": 1.0 / dt, "nbest": len(nb),
-                                      "best_score": float(nb[0].score),
+                                      "best_score": float(nb[0].score), "best_yseq": best["ref_eager"][0],
                                       "api": "the reference's own decoder + CTCPrefixScorer + BatchBeamSearch .to('cuda'), fp32 eager"}
         except Exception as e:                               # noqa: BLE001
             out["reference_eager"] = {"error": f"{type(e).__name__}: {e}"}

@@ -295,7 +295,7 @@ def test_ddp_gradient_allreduce_two_ranks(dev):
     DistributedDataParallel over a stack of the slice's modules -- every gradient is produced by libavsr_b200's backward
     and all-reduced by DDP's hooks on the original Parameters (train.py:37)."""
     if torch.cuda.device_count() < 2:
-        pytest.skip("needs 2 GPUs (gpurun --gpus 2)")
+        pytest.skip("needs 2 GPUs")
     import subprocess, sys
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
     r = subprocess.run([sys.executable, "-m", "torch.distributed.run", "--nnodes=1", "--nproc-per-node=2", "--master-addr",
