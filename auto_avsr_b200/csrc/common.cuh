@@ -48,8 +48,6 @@ extern std::atomic<uint64_t> g_launches;
     if (_r != AVSR_OK) return _r; \
   } while (0)
 
-constexpr int kSplitCounters = 4096;  // split-K tile counters a caller must provide (EpiParams::counters)
-constexpr int kMaxSplits = 8;         // split-K slices gemm_tc may choose; sizes EpiParams::partial
 constexpr int kHeadDim = 64;  // d_k of the reference encoder (768 / 12); the attention kernels are built for it
 
 static inline size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
@@ -60,14 +58,9 @@ static inline int cdiv(int a, int b) { return (a + b - 1) / b; }
 // scheduling, barrier init, TMEM allocation, tensor-map prefetch) while its predecessor in the stream / graph is
 // still draining, and blocks in pdl_wait() until the predecessor has completed and flushed before it touches any
 // global memory.  pdl_launch_dependents() at the top lets the successor do the same.  Without the attribute both
-// are no-ops, so the same kernels work under plain launches (AVSR_B200_PDL=0).
+// are no-ops, so the same kernels also work under plain <<<>>> launches.
 __device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
 __device__ __forceinline__ void pdl_launch_dependents() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
-
-inline bool pdl_enabled() {
-  static const bool on = [] { const char* e = getenv("AVSR_B200_PDL"); return !(e && e[0] == '0'); }();
-  return on;
-}
 
 template <typename... KArgs, typename... Args, size_t... I>
 inline cudaError_t launch_kernel_impl(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st,
@@ -80,7 +73,7 @@ inline cudaError_t launch_kernel_impl(void (*kernel)(KArgs...), dim3 grid, dim3 
   attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
   attr[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr;
-  cfg.numAttrs = pdl_enabled() ? 1 : 0;
+  cfg.numAttrs = 1;
   return cudaLaunchKernelExC(&cfg, reinterpret_cast<const void*>(kernel), ptrs);
 }
 // launch `kernel<<<grid, block, smem, st>>>(args...)` with the PDL attribute
@@ -217,8 +210,6 @@ struct EpiParams {
   int T, H, Tp, Rp;   // frames per utterance, heads, padded T of v^T, padded rows of the pos table
   const float* pos_u; // QK: [H*64]
   const float* pos_v;
-  float* partial;     // split-K: fp32 workspace [splits][M][ldo] for the partial tiles (deterministic fix-up)
-  int* counters;      // split-K: one arrival counter per output tile, zero on entry, reset by the last arriver
   int n_valid;        // LSE: columns >= n_valid are padding (stored, but excluded from the partials)
   LsePart* lse_part;  // LSE: [2 * tiles_n][M] partials (two epilogue warps per lane quarter split a tile's columns)
   void* qu;           // operand-typed (float for OP_F32/OP_TF32, __half for OP_F16)
@@ -348,14 +339,14 @@ int gemm_tc(int mode, int opk, const void* A, const void* Bw, int M, int N, int 
 int gemm_tc2_try(int mode, const void* A, const void* Bw, int M, int N, int K, const EpiParams& ep, cudaStream_t st,
                  int* handled);
 
-// deferred split-K (gemm_tc2.cu): plan returns 1 and fills bnp / nsplit when the shape qualifies; the GEMM writes
-// partial[s][M][N] (raw fp32 k-slice sums) and the consuming LayerNorm finishes the residual update (LnParts)
-int gemm_tc2_splitk_plan(int M, int N, int K, int* bnp, int* nsplit);
+// deferred split-K (gemm_tc2.cu): plan returns 1 and fills nsplit (= kW2Splits) when the shape qualifies; the GEMM
+// writes partial[s][M][N] (raw fp32 k-slice sums) and the consuming LayerNorm finishes the residual update (LnParts)
+constexpr int kW2Splits = 3;
+int gemm_tc2_splitk_plan(int M, int N, int K, int* nsplit);
 // true while the caller guarantees that B operands are prepared weights no kernel of the stream writes (the encoder
-// forward): lets the experimental AVSR_B200_PREB=1 variant fetch weights before griddepcontrol.wait
+// forward): the two-SM GEMM then fetches weights before griddepcontrol.wait
 extern thread_local bool g_tc2_weights_static;
-int gemm_tc2_splitk(const void* A, const void* Bw, int M, int N, int K, float* partial, int bnp, int nsplit,
-                    cudaStream_t st);
+int gemm_tc2_splitk(const void* A, const void* Bw, int M, int N, int K, float* partial, int nsplit, cudaStream_t st);
 
 // ctc_lo (gemm_tc2.cu): logits[M][ldo] = A Bw^T + bias (fp32; N a multiple of 512, padded columns included) and
 // part[nparts][M] log-sum-exp partials over the columns < n_valid; *nparts = 2 * N / 512.  Needs M >= 256, K % 64 == 0.

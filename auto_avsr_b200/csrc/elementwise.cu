@@ -34,11 +34,12 @@ int launch_embed_scale(const float* xs, float* x, long n, float scale, cudaStrea
 }
 
 // ------------------------------------------------------------------ LayerNorm (layer_norm.py:21, eps 1e-12)
-// A row (d <= 1024 channels) is held in registers by WPR warps (1, 2 or 4): HBM / L2 sees exactly one read and one
-// write per element.  Two-pass mean / centred variance; warp-shuffle reductions, combined across the row's warps
-// through shared memory in a fixed order (deterministic).  The r02 launch timeline showed these kernels to be bound by
-// the latency of one load -> reduce -> store chain per warp (1 600 warps on 148 SMs is a single, half-empty wave), so
-// the geometry is a launch parameter: more warps per row = shorter chains and more loads in flight per SM.
+// A row (d <= 1024 channels) is held in registers by WPR warps: HBM / L2 sees exactly one read and one write per
+// element.  Two-pass mean / centred variance; warp-shuffle reductions, combined across the row's warps through shared
+// memory in a fixed order (deterministic).  The r02 launch timeline showed these kernels to be bound by the latency of
+// one load -> reduce -> store chain per warp (1 600 warps on 148 SMs is a single, half-empty wave), so more warps per
+// row = shorter chains and more loads in flight per SM.  2 warps per row x 4 rows per CTA was best in situ (r02 sweep
+// of 1x8, 1x2, 2x4, 2x2, 4x2, 4x1: profiles/r02_ln_sweep.txt).
 //   TWO = false : y = LN(x; g1, b1)                                   (y in operand storage or fp32)
 //   TWO = true  : y1 = LN(x; g1, b1) (fp32, may alias x) and y = LN(y1; g2, b2) in operand storage -- layer l's
 //                 norm_final followed by layer l+1's norm_ff_macaron (conformer_encoder.py:161-162 then :113).
@@ -46,7 +47,8 @@ int launch_embed_scale(const float* xs, float* x, long n, float scale, cudaStrea
 //                 (bias + part[0] + ... + part[NP-1]), fixed order; the updated row is written to pp.x_out when that
 //                 is not already the kernel's own fp32 output.  All loads of the row are issued before the first use
 //                 and before any store (a store in between would serialise them: possible aliasing).
-constexpr int kLnMaxVec = 8;  // float4 per lane at WPR = 1: 8 * 32 lanes * 4 = 1024 channels
+constexpr int kLnWpr = 2, kLnRpc = 4;   // warps per row, rows per CTA
+constexpr int kLnMaxD = 1024;           // 4 float4 per lane at 2 warps per row
 
 __device__ __forceinline__ void ln_named_bar(int id, int nthreads) {
   asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(nthreads) : "memory");
@@ -189,56 +191,29 @@ ln_kernel(const float* x /* may alias y1 / pp.x_out */, const float* __restrict_
   AVSR_TSPAN_CLOSE();
 }
 
-// launch geometry: warps per row x rows per CTA.  AVSR_B200_LN="<wpr>x<rows>" overrides (1x8 = the round-1 kernel).
-struct LnGeom { int wpr, rpc; };
-static LnGeom ln_geom(int d) {
-  static const LnGeom env = [] {
-    LnGeom g{0, 0};
-    if (const char* e = getenv("AVSR_B200_LN")) { if (sscanf(e, "%dx%d", &g.wpr, &g.rpc) != 2) g = LnGeom{0, 0}; }
-    return g;
-  }();
-  LnGeom g = env.wpr ? env : LnGeom{2, 4};   // r02 sweep (profiles/r02_ln_sweep.txt): 2x4 best in situ
-  (void)d;
-  return g;
-}
-
 template <int NP, bool TWO>
 static int launch_ln_np(const float* x, const float* g1, const float* b1, const float* g2, const float* b2, float* y1,
                         void* y, int rows, int d, int out_kind, cudaStream_t st, const LnParts& pp) {
-  const LnGeom g = ln_geom(d);
-  // vectors per lane: the reference's d = 768 needs 6 / 3 / 2 at 1 / 2 / 4 warps per row; up to 1024 channels 8 / 4 / 2
-  const bool small = d <= 768;
-#define AVSR_LN_CASE(W, R, VS, VL)                                                                                  \
-  if (g.wpr == W && g.rpc == R) {                                                                                   \
-    if (small)                                                                                                      \
-      AVSR_LAUNCH((ln_kernel<NP, TWO, W, R, VS>), cdiv(rows, R), 32 * W * R, 0, st, x, g1, b1, g2, b2, y1, y, rows, \
-                  d, out_kind, pp);                                                                                 \
-    else                                                                                                            \
-      AVSR_LAUNCH((ln_kernel<NP, TWO, W, R, VL>), cdiv(rows, R), 32 * W * R, 0, st, x, g1, b1, g2, b2, y1, y, rows, \
-                  d, out_kind, pp);                                                                                 \
-    return AVSR_OK;                                                                                                 \
-  }
-  AVSR_LN_CASE(1, 8, 6, 8) AVSR_LN_CASE(1, 2, 6, 8)
-  AVSR_LN_CASE(2, 4, 3, 4) AVSR_LN_CASE(2, 2, 3, 4)
-  AVSR_LN_CASE(4, 2, 2, 2) AVSR_LN_CASE(4, 1, 2, 2)
-#undef AVSR_LN_CASE
-  AVSR_REQUIRE(false, "layernorm: geometry %dx%d not instantiated", g.wpr, g.rpc);
+  // vectors per lane: 3 for the reference's d = 768, 4 up to 1024 channels
+  if (d <= 768)
+    AVSR_LAUNCH((ln_kernel<NP, TWO, kLnWpr, kLnRpc, 3>), cdiv(rows, kLnRpc), 32 * kLnWpr * kLnRpc, 0, st, x, g1, b1, g2,
+                b2, y1, y, rows, d, out_kind, pp);
+  else
+    AVSR_LAUNCH((ln_kernel<NP, TWO, kLnWpr, kLnRpc, 4>), cdiv(rows, kLnRpc), 32 * kLnWpr * kLnRpc, 0, st, x, g1, b1, g2,
+                b2, y1, y, rows, d, out_kind, pp);
   return AVSR_OK;
 }
 
 template <bool TWO>
 static int launch_ln(const float* x, const float* g1, const float* b1, const float* g2, const float* b2, float* y1,
                      void* y, int rows, int d, int out_kind, cudaStream_t st, const LnParts* parts) {
-  AVSR_REQUIRE(d % 4 == 0 && d <= kLnMaxVec * 128 && d > 0, "layernorm: d=%d must be a multiple of 4 and <= %d", d,
-               kLnMaxVec * 128);
+  AVSR_REQUIRE(d % 4 == 0 && d <= kLnMaxD && d > 0, "layernorm: d=%d must be a multiple of 4 and <= %d", d, kLnMaxD);
   if (rows <= 0) return AVSR_OK;
   const LnParts pp = parts ? *parts : LnParts{};
   switch (pp.nparts) {
     case 0: return launch_ln_np<0, TWO>(x, g1, b1, g2, b2, y1, y, rows, d, out_kind, st, pp);
-    case 2: return launch_ln_np<2, TWO>(x, g1, b1, g2, b2, y1, y, rows, d, out_kind, st, pp);
-    case 3: return launch_ln_np<3, TWO>(x, g1, b1, g2, b2, y1, y, rows, d, out_kind, st, pp);
-    case 4: return launch_ln_np<4, TWO>(x, g1, b1, g2, b2, y1, y, rows, d, out_kind, st, pp);
-    default: AVSR_REQUIRE(false, "layernorm: %d k-slices not instantiated (0, 2, 3, 4)", pp.nparts);
+    case kW2Splits: return launch_ln_np<kW2Splits, TWO>(x, g1, b1, g2, b2, y1, y, rows, d, out_kind, st, pp);
+    default: AVSR_REQUIRE(false, "layernorm: %d k-slices not instantiated (0, %d)", pp.nparts, kW2Splits);
   }
   return AVSR_OK;
 }
@@ -309,9 +284,9 @@ int launch_sinusoid(void* pe, int T, int d, int out_kind, cudaStream_t st) {
 // shared memory for 8 outputs (the v1 kernel read 2 per output pair: 4x more shared-memory traffic, r01 profile).
 constexpr int kDwTT = 64;    // frames per CTA
 constexpr int kDwFr = 8;     // frames per thread
-// channels per CTA (CH) is a launch-time choice: 64 (16 quads, 128 threads, 336 CTAs at S2) or 32 (8 quads, 64 threads,
-// 672 CTAs: the same halo ratio and full 128-byte row segments, twice as many CTAs in flight per SM to hide the
-// load -> barrier -> compute -> store chain of each)
+// channels per CTA (CH): 32 for K = 31 (8 quads, 64 threads, 672 CTAs at S2: the same halo ratio as 64 and full
+// 128-byte row segments, with twice as many CTAs in flight per SM to hide the load -> barrier -> compute -> store chain
+// of each); 64 for the runtime-K kernel
 
 template <int K, int QPR>
 __device__ __forceinline__ void dw_accumulate(const float4* in_s, const float4* w_s, int q, int ts, int k_runtime,
@@ -430,11 +405,8 @@ int launch_dwconv_bn_silu(const float* x, const float* wt, const float* scale, c
                           int T, int C, int K, int out_kind, cudaStream_t st) {
   AVSR_REQUIRE(C % 4 == 0 && K % 2 == 1 && K >= 1 && K <= 255, "dwconv: C=%d must be a multiple of 4, K=%d odd", C, K);
   if (B <= 0 || T <= 0) return AVSR_OK;
-  static const int ch = [] { const char* e = getenv("AVSR_B200_DW"); return (e && atoi(e) == 64) ? 64 : 32; }();
-  if (K == 31) {   // the reference's cnn_module_kernel (e2e_asr_conformer.py:38): fully unrolled taps
-    return ch == 64 ? launch_dw<31, 64>(x, wt, scale, shift, y, B, T, C, K, out_kind, st)
-                    : launch_dw<31, 32>(x, wt, scale, shift, y, B, T, C, K, out_kind, st);
-  }
+  if (K == 31)   // the reference's cnn_module_kernel (e2e_asr_conformer.py:38): fully unrolled taps
+    return launch_dw<31, 32>(x, wt, scale, shift, y, B, T, C, K, out_kind, st);
   return launch_dw<0, 64>(x, wt, scale, shift, y, B, T, C, K, out_kind, st);
 }
 

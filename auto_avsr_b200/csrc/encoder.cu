@@ -146,11 +146,9 @@ static inline const void* op_offset(const void* base, size_t elems, int precisio
 }
 
 // ------------------------------------------------------------------ workspace
-constexpr int kMaxBranches = 4;   // a plan may run up to this many batch slices as concurrent graph branches
 struct Workspace {
   float *x, *xn, *hid, *qu, *qv, *kk, *vt, *ctx, *glu, *dw, *pe, *pos;
-  float* splitk;      // [kMaxSplits][N][d_model] fp32 partial tiles of the split-K residual GEMMs
-  int* counters;      // [kSplitCounters] tile arrival counters (zero between launches)
+  float* splitk;      // [kW2Splits][N][d_model] fp32 k-slices of the deferred FFN w_2 GEMM (gemm_tc2_splitk)
   int32_t* lengths;
   int Tp, Rp;
   size_t bytes;
@@ -168,26 +166,10 @@ static Workspace layout_workspace(const AvsrEncoderConfig& c, int B, int T, void
   W.ctx = cv.take(N * D); W.glu = cv.take(N * D); W.dw = cv.take(N * D);
   W.pe = cv.take((size_t)W.Rp * D);
   W.pos = cv.take((size_t)c.num_blocks * W.Rp * D);
-  W.splitk = cv.take((size_t)kMaxSplits * N * D);
-  W.counters = reinterpret_cast<int*>(cv.take((size_t)kSplitCounters * kMaxBranches));
+  W.splitk = cv.take((size_t)kW2Splits * N * D);
   W.lengths = reinterpret_cast<int32_t*>(cv.take((size_t)B));
   W.bytes = cv.off;
   return W;
-}
-
-// The view of batch elements [b0, b0 + ...) of a workspace laid out for the whole batch: every per-frame buffer is
-// row-major in (b, t), so a slice is a pointer offset (offsets are taken in floats also where a buffer holds halfs:
-// the slices stay disjoint and 16-byte aligned).  pe / pos depend on T only and are shared.
-static Workspace slice_workspace(const Workspace& W, const AvsrEncoderConfig& c, int b0, int T, int branch) {
-  Workspace S = W;
-  const size_t r = (size_t)b0 * T, D = c.d_model, F = c.linear_units;
-  S.x += r * D; S.xn += r * D; S.hid += r * F; S.qu += r * D; S.qv += r * D; S.kk += r * D;
-  S.vt += (size_t)b0 * D * W.Tp;
-  S.ctx += r * D; S.glu += r * D; S.dw += r * D;
-  S.splitk += (size_t)kMaxSplits * r * D;
-  S.counters += (size_t)branch * kSplitCounters;
-  S.lengths += b0;
-  return S;
 }
 
 __global__ void fill_lengths_kernel(int32_t* dst, const int32_t* src, int B, int T) {
@@ -234,14 +216,6 @@ static EpiParams epi_linear(int M, int N, const float* bias, void* out, const fl
   return e;
 }
 
-// residual-stream GEMM: x += alpha * (A W^T + b); may be split along K (deterministic fix-up through `W.splitk`)
-static EpiParams epi_resid(int M, int N, const float* bias, float* x, float alpha, float* splitk, int* counters) {
-  EpiParams e = epi_linear(M, N, bias, x, x, alpha, 0, 0);
-  e.partial = splitk;
-  e.counters = counters;
-  return e;
-}
-
 static int run_gemm(int prec, int mode, const void* A, const void* Bw, int M, int N, int K, const EpiParams& e,
                     cudaStream_t st) {
   if (prec == AVSR_PREC_FP32)
@@ -268,10 +242,9 @@ static int compute_pos(const AvsrEncoderConfig& c, const Prepared& P, const Work
   return run_gemm(prec, EPI_POS, W.pe, P.pos_w_all, W.Rp, L * D, D, e, ps);
 }
 
-// pos_external: the caller computes the pos tables (compute_pos) and records aux->join; this body only waits for it
 static int forward_body(const AvsrEncoderConfig& c, const Prepared& P, const Workspace& W, int B, int T,
                         const int32_t* lengths, float* taps, int prec, cudaStream_t st, const AuxFork* aux = nullptr,
-                        bool pos_external = false, unsigned long long* sat = nullptr) {
+                        unsigned long long* sat = nullptr) {
   const int N = B * T, D = c.d_model, F = c.linear_units, H = c.n_heads, L = c.num_blocks;
   const int opk = operand_kind(prec);           // storage of every tensor that feeds a contraction
   const int opr = prec != AVSR_PREC_FP32;       // "destination is operand-typed" flag of the epilogues
@@ -283,9 +256,7 @@ static int forward_body(const AvsrEncoderConfig& c, const Prepared& P, const Wor
     ~StaticWeights() { g_tc2_weights_static = false; }
   } static_weights_scope;
 
-  // split-K tile counters must be zero on entry (they re-arm themselves; this covers a first use / an aborted run)
-  AVSR_CUDA_TRY(cudaMemsetAsync(W.counters, 0, kSplitCounters * sizeof(int), st));
-  if (!pos_external) {
+  {
     cudaStream_t ps = st;
     if (aux) {
       AVSR_CUDA_TRY(cudaEventRecord(aux->fork, st));
@@ -301,8 +272,8 @@ static int forward_body(const AvsrEncoderConfig& c, const Prepared& P, const Wor
 
   // FFN w_2 (K = linear_units) as a deferred split-K GEMM: k-slices land in W.splitk and the LayerNorm that follows
   // applies x += 0.5 * (sum of slices + b) while it loads the row.  Not with `taps` (they read x between the two).
-  int w2_bnp = 0, w2_split = 0;
-  const bool w2_defer = prec == AVSR_PREC_F16 && !taps && gemm_tc2_splitk_plan(N, D, F, &w2_bnp, &w2_split);
+  int w2_split = 0;
+  const bool w2_defer = prec == AVSR_PREC_F16 && !taps && gemm_tc2_splitk_plan(N, D, F, &w2_split);
   auto w2_parts = [&](const float* bias, float* x_out) {
     LnParts pp;
     pp.part = W.splitk; pp.nparts = w2_split; pp.stride = (long)N * D; pp.bias = bias; pp.alpha = 0.5f; pp.x_out = x_out;
@@ -323,9 +294,9 @@ static int forward_body(const AvsrEncoderConfig& c, const Prepared& P, const Wor
     AVSR_TRY(run_gemm(prec, EPI_LINEAR, W.xn, w.ffm_w1, N, F, D, epi_linear(N, F, w.ffm_b1, W.hid, nullptr, 0.f, 1, opr), st));
     AVSR_TRY(chk(W.hid, (size_t)N * F));
     if (w2_defer) {
-      AVSR_TRY(gemm_tc2_splitk(W.hid, w.ffm_w2, N, D, F, W.splitk, w2_bnp, w2_split, st));
+      AVSR_TRY(gemm_tc2_splitk(W.hid, w.ffm_w2, N, D, F, W.splitk, w2_split, st));
     } else {
-      AVSR_TRY(run_gemm(prec, EPI_LINEAR, W.hid, w.ffm_w2, N, D, F, epi_resid(N, D, w.ffm_b2, W.x, 0.5f, W.splitk, W.counters), st));
+      AVSR_TRY(run_gemm(prec, EPI_LINEAR, W.hid, w.ffm_w2, N, D, F, epi_linear(N, D, w.ffm_b2, W.x, W.x, 0.5f, 0, 0), st));
       AVSR_TRY(tap(0));
     }
     // (2) rel-pos MHA: x += out(attn(LN(x)))                                  conformer_encoder.py:119-142
@@ -365,7 +336,7 @@ static int forward_body(const AvsrEncoderConfig& c, const Prepared& P, const Wor
         AVSR_TRY(attention_simt(W.qu, W.qv, W.kk, W.vt, (const float*)pos_l, lengths, W.ctx, B, T, H, W.Tp, W.Rp, 0, st));
     }
     AVSR_TRY(chk(W.ctx, (size_t)N * D));
-    AVSR_TRY(run_gemm(prec, EPI_LINEAR, W.ctx, w.out_w, N, D, D, epi_resid(N, D, w.out_b, W.x, 1.0f, W.splitk, W.counters), st));
+    AVSR_TRY(run_gemm(prec, EPI_LINEAR, W.ctx, w.out_w, N, D, D, epi_linear(N, D, w.out_b, W.x, W.x, 1.0f, 0, 0), st));
     AVSR_TRY(tap(1));
     // (3) conv module: x += pw2(silu(bn(dw(glu(pw1 LN(x))))))                 conformer_encoder.py:145-151, :30-35
     AVSR_TRY(launch_layernorm(W.x, w.ln_conv_w, w.ln_conv_b, W.xn, N, D, opk, st));
@@ -377,7 +348,7 @@ static int forward_body(const AvsrEncoderConfig& c, const Prepared& P, const Wor
     }
     AVSR_TRY(launch_dwconv_bn_silu(W.glu, w.dw_wt, w.dw_scale, w.dw_shift, W.dw, B, T, D, c.cnn_kernel, opk, st));
     AVSR_TRY(chk(W.dw, (size_t)N * D));
-    AVSR_TRY(run_gemm(prec, EPI_LINEAR, W.dw, w.pw2_w, N, D, D, epi_resid(N, D, w.pw2_b, W.x, 1.0f, W.splitk, W.counters), st));
+    AVSR_TRY(run_gemm(prec, EPI_LINEAR, W.dw, w.pw2_w, N, D, D, epi_linear(N, D, w.pw2_b, W.x, W.x, 1.0f, 0, 0), st));
     AVSR_TRY(tap(2));
     // (4) FFN: x += 0.5 * w2(relu(w1 LN(x)))                                  conformer_encoder.py:154-159
     AVSR_TRY(launch_layernorm(W.x, w.ln_ff_w, w.ln_ff_b, W.xn, N, D, opk, st));
@@ -385,9 +356,9 @@ static int forward_body(const AvsrEncoderConfig& c, const Prepared& P, const Wor
     AVSR_TRY(run_gemm(prec, EPI_LINEAR, W.xn, w.ff_w1, N, F, D, epi_linear(N, F, w.ff_b1, W.hid, nullptr, 0.f, 1, opr), st));
     AVSR_TRY(chk(W.hid, (size_t)N * F));
     if (w2_defer) {
-      AVSR_TRY(gemm_tc2_splitk(W.hid, w.ff_w2, N, D, F, W.splitk, w2_bnp, w2_split, st));
+      AVSR_TRY(gemm_tc2_splitk(W.hid, w.ff_w2, N, D, F, W.splitk, w2_split, st));
     } else {
-      AVSR_TRY(run_gemm(prec, EPI_LINEAR, W.hid, w.ff_w2, N, D, F, epi_resid(N, D, w.ff_b2, W.x, 0.5f, W.splitk, W.counters), st));
+      AVSR_TRY(run_gemm(prec, EPI_LINEAR, W.hid, w.ff_w2, N, D, F, epi_linear(N, D, w.ff_b2, W.x, W.x, 0.5f, 0, 0), st));
       AVSR_TRY(tap(3));
     }
     // (5) x = LN_final(x)                                                     conformer_encoder.py:161-162
@@ -426,20 +397,9 @@ static int forward_impl(const AvsrEncoderConfig* cfg, const void* prepared, cons
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
   AVSR_TRY(launch_embed_scale(xs, W.x, (long)B * T * cfg->d_model, sqrtf((float)cfg->d_model), st));
   if (sat) AVSR_CUDA_TRY(cudaMemsetAsync(sat, 0, sizeof(unsigned long long), st));
-  AVSR_TRY(forward_body(*cfg, P, W, B, T, lengths, taps, precision, st, nullptr, false, sat));
+  AVSR_TRY(forward_body(*cfg, P, W, B, T, lengths, taps, precision, st, nullptr, sat));
   AVSR_TRY(launch_layernorm(W.x, P.after_w, P.after_b, out, B * T, cfg->d_model, 0, st));
   return AVSR_OK;
-}
-
-// How many batch slices a plan runs as concurrent graph branches.  AVSR_B200_BRANCHES overrides (1 = off).
-static int plan_branches(int B, int T, int precision) {
-  int want = 1;
-  if (const char* e = getenv("AVSR_B200_BRANCHES")) want = atoi(e);
-  if (precision != AVSR_PREC_F16 || want < 2) return 1;
-  if (want > kMaxBranches) want = kMaxBranches;
-  if (want > B) want = B;
-  while (want > 1 && (long)(B / want) * T < 256) --want;   // every slice must still feed the two-SM GEMMs (M >= 256)
-  return want;
 }
 
 // ------------------------------------------------------------------ the steps either side of the encoder (SURVEY 8f #1)
@@ -533,7 +493,70 @@ struct AvsrPlan {
   int head_idim = 0;
   cudaGraph_t graph = nullptr;
   cudaGraphExec_t exec = nullptr;
+  uint64_t kernel_nodes = 0;       // launches one replay adds to avsr_launch_count
 };
+
+static uint64_t graph_kernel_nodes(cudaGraph_t g) {
+  size_t n = 0;
+  if (cudaGraphGetNodes(g, nullptr, &n) != cudaSuccess) return 0;
+  std::vector<cudaGraphNode_t> nodes(n);
+  if (n == 0 || cudaGraphGetNodes(g, nodes.data(), &n) != cudaSuccess) return 0;
+  uint64_t k = 0;
+  for (auto nd : nodes) {
+    cudaGraphNodeType t;
+    if (cudaGraphNodeGetType(nd, &t) == cudaSuccess && t == cudaGraphNodeTypeKernel) ++k;
+  }
+  return k;
+}
+
+// Records `body(aux)` -- the schedule on `st`, with the rel-pos branch forked onto `aux` -- into p->graph / p->exec.
+// The body runs once outside capture first (function attributes such as the dynamic shared-memory opt-in must not be
+// set lazily during capture; lazy module loading), then is captured; the captured launches are counted when the graph
+// is replayed.  The auxiliary stream and events live for the duration of the call.  On error nothing is left behind
+// but `p` itself, which the caller deletes.
+template <typename Body>
+static int capture_plan(AvsrPlan* p, cudaStream_t st, Body&& body) {
+  AuxFork aux;
+  int rc = AVSR_OK;
+  if (cudaStreamCreateWithFlags(&aux.stream, cudaStreamNonBlocking) != cudaSuccess ||
+      cudaEventCreateWithFlags(&aux.fork, cudaEventDisableTiming) != cudaSuccess ||
+      cudaEventCreateWithFlags(&aux.join, cudaEventDisableTiming) != cudaSuccess) {
+    set_error("plan: cannot create the auxiliary stream / events: %s", cudaGetErrorString(cudaGetLastError()));
+    rc = AVSR_E_CUDA;
+  }
+  if (rc == AVSR_OK) rc = body(&aux);
+  if (rc == AVSR_OK && (cudaStreamSynchronize(st) != cudaSuccess || cudaStreamSynchronize(aux.stream) != cudaSuccess)) {
+    set_error("plan warm-up failed: %s", cudaGetErrorString(cudaGetLastError()));
+    rc = AVSR_E_CUDA;
+  }
+  if (rc == AVSR_OK) {
+    cudaError_t e = cudaStreamBeginCapture(st, cudaStreamCaptureModeThreadLocal);
+    if (e != cudaSuccess) {
+      set_error("cudaStreamBeginCapture: %s", cudaGetErrorString(e));
+      rc = AVSR_E_CUDA;
+    } else {
+      const uint64_t before = g_launches.load();
+      rc = body(&aux);   // the aux stream joins the capture through the fork event
+      g_launches.store(before);
+      e = cudaStreamEndCapture(st, &p->graph);
+      if (rc == AVSR_OK && e != cudaSuccess) { set_error("cudaStreamEndCapture: %s", cudaGetErrorString(e)); rc = AVSR_E_CUDA; }
+    }
+  }
+  if (rc == AVSR_OK) {
+    const cudaError_t e = cudaGraphInstantiate(&p->exec, p->graph, 0);
+    if (e != cudaSuccess) { set_error("cudaGraphInstantiate: %s", cudaGetErrorString(e)); rc = AVSR_E_CUDA; }
+  }
+  if (aux.join) cudaEventDestroy(aux.join);
+  if (aux.fork) cudaEventDestroy(aux.fork);
+  if (aux.stream) cudaStreamDestroy(aux.stream);
+  if (rc != AVSR_OK) {
+    if (p->graph) cudaGraphDestroy(p->graph);
+    p->graph = nullptr;
+    return rc;
+  }
+  p->kernel_nodes = graph_kernel_nodes(p->graph);
+  return AVSR_OK;
+}
 
 #ifdef AVSR_TRACE
 namespace avsr {
@@ -662,91 +685,14 @@ int avsr_plan_create(const AvsrEncoderConfig* cfg, const void* prepared, int B, 
   p->cfg = *cfg; p->B = B; p->T = T; p->precision = precision; p->W = W;
   p->P = layout_prepared(*cfg, const_cast<void*>(prepared));
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
-  // warm-up outside capture: sets function attributes (dynamic smem opt-in) that capture must not do lazily
   fill_lengths_kernel<<<cdiv(B, 128), 128, 0, st>>>(W.lengths, nullptr, B, T);
   g_launches.fetch_add(1);
-  AuxFork aux;
-  if (cudaStreamCreateWithFlags(&aux.stream, cudaStreamNonBlocking) != cudaSuccess ||
-      cudaEventCreateWithFlags(&aux.fork, cudaEventDisableTiming) != cudaSuccess ||
-      cudaEventCreateWithFlags(&aux.join, cudaEventDisableTiming) != cudaSuccess) {
-    set_error("plan: cannot create the auxiliary stream / events: %s", cudaGetErrorString(cudaGetLastError()));
-    delete p;
-    return AVSR_E_CUDA;
-  }
-  auto drop_aux0 = [&]() {
-    cudaEventDestroy(aux.fork); cudaEventDestroy(aux.join); cudaStreamDestroy(aux.stream);
-  };
-  // Batch slices as concurrent branches (frames of different batch elements never interact in this path): the GEMMs
-  // of one slice fill the SMs another slice's one-tile-per-cluster kernels leave idle and hide their un-overlapped
-  // prologues / epilogues.  Slice h covers batch elements [b0_h, b0_h + B_h); slice 0 runs on the caller's stream.
-  const int nbr = plan_branches(B, T, precision);
-  std::vector<cudaStream_t> bstream(nbr, st);
-  std::vector<cudaEvent_t> bdone(nbr, nullptr);
-  bool bok = true;
-  for (int h = 1; h < nbr; ++h)
-    bok = bok && cudaStreamCreateWithFlags(&bstream[h], cudaStreamNonBlocking) == cudaSuccess &&
-          cudaEventCreateWithFlags(&bdone[h], cudaEventDisableTiming) == cudaSuccess;
-  auto drop_aux = [&]() {
-    drop_aux0();
-    for (int h = 1; h < nbr; ++h) { if (bdone[h]) cudaEventDestroy(bdone[h]); if (bstream[h] != st) cudaStreamDestroy(bstream[h]); }
-  };
-  if (!bok) { set_error("plan: cannot create the branch streams"); drop_aux(); delete p; return AVSR_E_CUDA; }
-  auto run_all = [&]() -> int {
-    if (nbr == 1) return forward_body(p->cfg, p->P, p->W, B, T, W.lengths, nullptr, precision, st, &aux);
-    AVSR_CUDA_TRY(cudaEventRecord(aux.fork, st));
-    AVSR_CUDA_TRY(cudaStreamWaitEvent(aux.stream, aux.fork, 0));
-    AVSR_TRY(compute_pos(p->cfg, p->P, p->W, T, precision, aux.stream));
-    AVSR_CUDA_TRY(cudaEventRecord(aux.join, aux.stream));
-    int b0 = 0;
-    for (int h = 0; h < nbr; ++h) {
-      const int Bh = B / nbr + (h < B % nbr ? 1 : 0);
-      if (h) AVSR_CUDA_TRY(cudaStreamWaitEvent(bstream[h], aux.fork, 0));
-      const Workspace Wh = slice_workspace(p->W, p->cfg, b0, T, h);
-      AVSR_TRY(forward_body(p->cfg, p->P, Wh, Bh, T, Wh.lengths, nullptr, precision, bstream[h], &aux, true));
-      if (h) {
-        AVSR_CUDA_TRY(cudaEventRecord(bdone[h], bstream[h]));
-        AVSR_CUDA_TRY(cudaStreamWaitEvent(st, bdone[h], 0));
-      }
-      b0 += Bh;
-    }
-    return AVSR_OK;
-  };
-  int rc = run_all();
-  if (rc == AVSR_OK) {
-    bool ok = cudaStreamSynchronize(st) == cudaSuccess && cudaStreamSynchronize(aux.stream) == cudaSuccess;
-    for (int h = 1; h < nbr; ++h) ok = ok && cudaStreamSynchronize(bstream[h]) == cudaSuccess;
-    if (!ok) { set_error("plan warm-up failed: %s", cudaGetErrorString(cudaGetLastError())); rc = AVSR_E_CUDA; }
-  }
-  if (rc != AVSR_OK) { drop_aux(); delete p; return rc; }
-  cudaError_t e = cudaStreamBeginCapture(st, cudaStreamCaptureModeThreadLocal);
-  if (e != cudaSuccess) { set_error("cudaStreamBeginCapture: %s", cudaGetErrorString(e)); drop_aux(); delete p; return AVSR_E_CUDA; }
-  const uint64_t before = g_launches.load();
-  rc = run_all();   // aux and the branch streams join the capture
-  g_launches.store(before);  // captured launches are counted when the graph is replayed
-  e = cudaStreamEndCapture(st, &p->graph);
-  drop_aux();
-  if (rc != AVSR_OK) { if (p->graph) cudaGraphDestroy(p->graph); delete p; return rc; }
-  if (e != cudaSuccess) { set_error("cudaStreamEndCapture: %s", cudaGetErrorString(e)); delete p; return AVSR_E_CUDA; }
-  e = cudaGraphInstantiate(&p->exec, p->graph, 0);
-  if (e != cudaSuccess) {
-    set_error("cudaGraphInstantiate: %s", cudaGetErrorString(e));
-    cudaGraphDestroy(p->graph); delete p; return AVSR_E_CUDA;
-  }
+  const int rc = capture_plan(p, st, [&](const AuxFork* aux) {
+    return forward_body(p->cfg, p->P, p->W, B, T, p->W.lengths, nullptr, precision, st, aux);
+  });
+  if (rc != AVSR_OK) { delete p; return rc; }
   *plan = p;
   return AVSR_OK;
-}
-
-static uint64_t graph_kernel_nodes(cudaGraph_t g) {
-  size_t n = 0;
-  if (cudaGraphGetNodes(g, nullptr, &n) != cudaSuccess) return 0;
-  std::vector<cudaGraphNode_t> nodes(n);
-  if (n == 0 || cudaGraphGetNodes(g, nodes.data(), &n) != cudaSuccess) return 0;
-  uint64_t k = 0;
-  for (auto nd : nodes) {
-    cudaGraphNodeType t;
-    if (cudaGraphNodeGetType(nd, &t) == cudaSuccess && t == cudaGraphNodeTypeKernel) ++k;
-  }
-  return k;
 }
 
 int avsr_plan_forward(AvsrPlan* p, const float* xs, const int32_t* lengths, float* out, void* stream) {
@@ -757,10 +703,7 @@ int avsr_plan_forward(AvsrPlan* p, const float* xs, const int32_t* lengths, floa
   AVSR_CHECK_LAUNCH();
   AVSR_TRY(launch_embed_scale(xs, p->W.x, (long)N * D, sqrtf((float)D), st));
   AVSR_CUDA_TRY(cudaGraphLaunch(p->exec, st));
-  static thread_local cudaGraph_t counted = nullptr;
-  static thread_local uint64_t nk = 0;
-  if (counted != p->graph) { nk = graph_kernel_nodes(p->graph); counted = p->graph; }
-  g_launches.fetch_add(nk);
+  g_launches.fetch_add(p->kernel_nodes);
   AVSR_TRY(launch_layernorm(p->W.x, p->P.after_w, p->P.after_b, out, N, D, 0, st));
   return AVSR_OK;
 }
@@ -1062,39 +1005,11 @@ int avsr_head_plan_create(const AvsrEncoderConfig* cfg, const void* prepared, co
   fill_lengths_kernel<<<cdiv(B, 128), 128, 0, st>>>(p->W.lengths, nullptr, B, T);
   g_launches.fetch_add(1);
   AVSR_CUDA_TRY(cudaMemsetAsync(feats_static, 0, (size_t)B * T * idim * sizeof(float), st));
-  AuxFork aux;
-  if (cudaStreamCreateWithFlags(&aux.stream, cudaStreamNonBlocking) != cudaSuccess ||
-      cudaEventCreateWithFlags(&aux.fork, cudaEventDisableTiming) != cudaSuccess ||
-      cudaEventCreateWithFlags(&aux.join, cudaEventDisableTiming) != cudaSuccess) {
-    set_error("plan: cannot create the auxiliary stream / events: %s", cudaGetErrorString(cudaGetLastError()));
-    delete p;
-    return AVSR_E_CUDA;
-  }
-  auto drop_aux = [&]() { cudaEventDestroy(aux.fork); cudaEventDestroy(aux.join); cudaStreamDestroy(aux.stream); };
-  auto run_all = [&]() -> int {
+  const int rc = capture_plan(p, st, [&](const AuxFork* aux) {
     return head_forward_body(p->cfg, p->P, H, p->W, HW, feats_static, p->W.lengths, B, T, idim, odim, enc_out, logp, argmax,
-                             precision, st, &aux);
-  };
-  int rc = run_all();     // warm-up outside capture (function attributes, lazy module loading)
-  if (rc == AVSR_OK && (cudaStreamSynchronize(st) != cudaSuccess || cudaStreamSynchronize(aux.stream) != cudaSuccess)) {
-    set_error("plan warm-up failed: %s", cudaGetErrorString(cudaGetLastError()));
-    rc = AVSR_E_CUDA;
-  }
-  if (rc != AVSR_OK) { drop_aux(); delete p; return rc; }
-  cudaError_t e = cudaStreamBeginCapture(st, cudaStreamCaptureModeThreadLocal);
-  if (e != cudaSuccess) { set_error("cudaStreamBeginCapture: %s", cudaGetErrorString(e)); drop_aux(); delete p; return AVSR_E_CUDA; }
-  const uint64_t before = g_launches.load();
-  rc = run_all();
-  g_launches.store(before);
-  e = cudaStreamEndCapture(st, &p->graph);
-  drop_aux();
-  if (rc != AVSR_OK) { if (p->graph) cudaGraphDestroy(p->graph); delete p; return rc; }
-  if (e != cudaSuccess) { set_error("cudaStreamEndCapture: %s", cudaGetErrorString(e)); delete p; return AVSR_E_CUDA; }
-  e = cudaGraphInstantiate(&p->exec, p->graph, 0);
-  if (e != cudaSuccess) {
-    set_error("cudaGraphInstantiate: %s", cudaGetErrorString(e));
-    cudaGraphDestroy(p->graph); delete p; return AVSR_E_CUDA;
-  }
+                             precision, st, aux);
+  });
+  if (rc != AVSR_OK) { delete p; return rc; }
   *plan = p;
   return AVSR_OK;
 }
@@ -1106,7 +1021,7 @@ int avsr_head_plan_forward(AvsrPlan* p, const float* feats, const int32_t* lengt
   AVSR_CHECK_LAUNCH();
   AVSR_CUDA_TRY(cudaMemcpyAsync(p->head_feats, feats, (size_t)p->B * p->T * p->head_idim * sizeof(float), cudaMemcpyDeviceToDevice, st));
   AVSR_CUDA_TRY(cudaGraphLaunch(p->exec, st));
-  g_launches.fetch_add(graph_kernel_nodes(p->graph));
+  g_launches.fetch_add(p->kernel_nodes);
   return AVSR_OK;
 }
 

@@ -111,7 +111,7 @@ template <> struct OpTraits<__half> {
 template <int MODE, int BN, int MSUB, typename TOp>
 __global__ void __launch_bounds__(TC_THREADS, 1)
 gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB, int K, int tiles_m,
-               int tiles_n, int splits, EpiParams ep) {
+               int tiles_n, EpiParams ep) {
   // PERSISTENT: CTA c processes tiles c, c + gridDim.x, ... (n fastest, so concurrently running CTAs share A rows in
   // L2).  The TMA ring never drains between tiles and the accumulator is double-buffered in TMEM, so the epilogue of
   // tile i overlaps the main loop of tile i+1 (at K = 768 a tile is only 12 k-blocks: per-tile prologue / pipeline
@@ -127,7 +127,6 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
   uint8_t* gen = tc_smem_raw + (base - raw);
   const uint32_t bars = base + S * Cfg::kStageBytes;  // full[S], empty[S], tmem_full[2], tmem_empty[2]
   uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(gen + S * Cfg::kStageBytes + (2 * S + 4) * 8);
-  uint32_t* s_flag = tmem_slot + 1;                                             // split-K: "this CTA arrived last"
   float* s_vec = reinterpret_cast<float*>(gen + S * Cfg::kStageBytes + 256);   // [3][BN]
   uint8_t* stg_base = gen + S * Cfg::kStageBytes + 256 + Cfg::kVecBytes;
   auto full_bar = [&](int s) { return bars + 8u * s; };
@@ -138,9 +137,6 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int nkb = K / KE;
   const int total_tiles = tiles_m * tiles_n;
-  // split-K (LINEAR into the residual stream only): work item = (tile, K-slice); slice-major order so that CTAs
-  // running at the same time reduce into different tiles.  Partial sums are added with red.global.add.v4.f32.
-  const int total_items = total_tiles * splits;
 
   pdl_launch_dependents();
   AVSR_TSPAN_OPEN(400 + MODE, (unsigned)BN | ((unsigned)MSUB << 16));
@@ -164,11 +160,9 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
   if (warp == 0) {
     {
       int it = 0;                                       // running k-block counter across tiles
-      for (int item = blockIdx.x; item < total_items; item += gridDim.x) {
-        const int tile = item % total_tiles, split = item / total_tiles;
+      for (int tile = blockIdx.x; tile < total_tiles; tile += gridDim.x) {
         const int m0 = (tile / tiles_n) * (TC_BM * MSUB), n0 = (tile % tiles_n) * BN;
-        const int kb0 = split * nkb / splits, kb1 = (split + 1) * nkb / splits;
-        for (int kb = kb0; kb < kb1; ++kb, ++it) {
+        for (int kb = 0; kb < nkb; ++kb, ++it) {
           const int s = it % S;
           const uint32_t ph = (it / S) & 1;
           mbar_wait(empty_bar(s), ph ^ 1);
@@ -187,15 +181,13 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
     {
       const uint32_t idesc = Op::idesc(TC_BM, BN);
       int it = 0, t = 0;
-      for (int item = blockIdx.x; item < total_items; item += gridDim.x, ++t) {
-        const int split = item / total_tiles;
-        const int kb0 = split * nkb / splits, kb1 = (split + 1) * nkb / splits;
+      for (int tile = blockIdx.x; tile < total_tiles; tile += gridDim.x, ++t) {
         const int acc = (ACC == 2) ? (t & 1) : 0;
         const uint32_t acc_ph = ((ACC == 2) ? (t >> 1) : t) & 1;
         mbar_wait(tmem_empty_bar(acc), acc_ph ^ 1);     // the epilogue has drained this accumulator
         tc_fence_after();
         const uint32_t tacc = tmem_base + acc * (MSUB * BN);
-        for (int kb = kb0; kb < kb1; ++kb, ++it) {
+        for (int kb = 0; kb < nkb; ++kb, ++it) {
           const int s = it % S;
           const uint32_t ph = (it / S) & 1;
           mbar_wait(full_bar(s), ph);
@@ -208,10 +200,10 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
               const uint64_t a_desc = umma_desc_sw128(a_addr + ms * (TC_BM * 128));
 #pragma unroll
               for (int k = 0; k < 4; ++k)  // one MMA-K = 32 bytes = +2 in the descriptor's 16-byte address field
-                Op::mma(tacc + ms * BN, a_desc + 2 * k, b_desc + 2 * k, idesc, (kb != kb0) || (k != 0));
+                Op::mma(tacc + ms * BN, a_desc + 2 * k, b_desc + 2 * k, idesc, (kb != 0) || (k != 0));
             }
             tc_commit(empty_bar(s));
-            if (kb == kb1 - 1) tc_commit(tmem_full_bar(acc));
+            if (kb == nkb - 1) tc_commit(tmem_full_bar(acc));
           }
         }
       }
@@ -227,8 +219,7 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
     constexpr int ONE = 16 / (int)sizeof(TOp);               // operand elements per 16-byte piece
     int t = 0;
 #pragma unroll 1
-    for (int item = blockIdx.x; item < total_items; item += gridDim.x, ++t) {
-    const int tile = item % total_tiles, split = item / total_tiles;
+    for (int tile = blockIdx.x; tile < total_tiles; tile += gridDim.x, ++t) {
     const int m0 = (tile / tiles_n) * (TC_BM * MSUB), n0 = (tile % tiles_n) * BN;
     const int acc = (ACC == 2) ? (t & 1) : 0;
     const uint32_t acc_ph = ((ACC == 2) ? (t >> 1) : t) & 1;
@@ -285,24 +276,11 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
             tmem_ld32(trow + c, v);
             tmem_ld_wait();
             const float* sb = s_vec + c;
-            if (splits == 1) {
 #pragma unroll
-              for (int j = 0; j < 32; ++j) { v[j] += sb[j]; if (ep.relu) v[j] = fmaxf(v[j], 0.f); }
-            }
+            for (int j = 0; j < 32; ++j) { v[j] += sb[j]; if (ep.relu) v[j] = fmaxf(v[j], 0.f); }
             stage_write_f32(stg, lane, v, false);
             __syncwarp();
             const int n = n0 + c + pc * 4;
-            if (splits > 1) {
-              // split-K: this K-slice's raw partial tile goes to the fp32 workspace (coalesced 16-byte stores); the
-              // last CTA to arrive for this tile sums the slices in fixed order (below) -> deterministic
-              float* part = ep.partial + (long)split * ep.M * ep.ldo;
-#pragma unroll
-              for (int it = 0; it < 8; ++it) {
-                const int m = mw + it * 4 + pr;
-                const uint4 pay = stage_read(stg, it, lane);
-                if (m < ep.M && n < ep.N) *reinterpret_cast<uint4*>(part + (long)m * ep.ldo + n) = pay;
-              }
-            } else {
             // residual pieces first (8 independent coalesced loads in flight), then combine + store: a load may not
             // be hoisted above a store by the compiler (possible aliasing), so the order is made explicit here
             float4 r[8];
@@ -325,7 +303,6 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
               }
               if (m < ep.M && n < ep.N)
                 *reinterpret_cast<float4*>(reinterpret_cast<float*>(ep.out) + (long)m * ep.ldo + n) = o;
-            }
             }
             __syncwarp();
           }
@@ -432,59 +409,6 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
     tc_fence_before();
     __syncwarp();
     if (lane == 0) mbar_arrive(tmem_empty_bar(acc));
-    if constexpr (MODE == EPI_LINEAR) {
-      if (splits > 1) {
-        // ---- deterministic split-K fix-up ("last block reduces"): publish the partial, count arrivals per tile ----
-        __threadfence();
-        asm volatile("bar.sync 1, 256;" ::: "memory");
-        if (threadIdx.x == 64) {
-          const int old = atomicAdd(ep.counters + tile, 1);
-          const int last = (old == splits - 1);
-          if (last) ep.counters[tile] = 0;                 // every slice has arrived: re-arm for the next launch
-          *s_flag = last;
-        }
-        asm volatile("bar.sync 1, 256;" ::: "memory");
-        if (*s_flag) {
-          __threadfence();                                 // acquire: the other slices' partial tiles are visible
-#pragma unroll 1
-          for (int ms = 0; ms < MSUB; ++ms) {
-            const int mw = m0 + ms * TC_BM + q * 32;
-#pragma unroll 1
-            for (int c = cb; c < ce; c += 32) {
-              const int n = n0 + c + pc * 4;
-              const float4 bv = *reinterpret_cast<const float4*>(s_vec + c + pc * 4);
-              // loads first (8 independent 16-byte loads in flight per slice, no store in between), stores last
-              float4 a[8], t4[8];
-              bool ok[8];
-#pragma unroll
-              for (int it = 0; it < 8; ++it) { a[it] = bv; ok[it] = (mw + it * 4 + pr < ep.M) && (n < ep.N); }
-              for (int sp = 0; sp < splits; ++sp) {        // fixed order: slice 0, 1, ... regardless of arrival order
-                const float* part = ep.partial + (long)sp * ep.M * ep.ldo;
-#pragma unroll
-                for (int it = 0; it < 8; ++it)
-                  t4[it] = ok[it] ? __ldcg(reinterpret_cast<const float4*>(part + (long)(mw + it * 4 + pr) * ep.ldo + n))
-                                  : make_float4(0.f, 0.f, 0.f, 0.f);
-#pragma unroll
-                for (int it = 0; it < 8; ++it) { a[it].x += t4[it].x; a[it].y += t4[it].y; a[it].z += t4[it].z; a[it].w += t4[it].w; }
-              }
-#pragma unroll
-              for (int it = 0; it < 8; ++it)
-                t4[it] = ok[it] ? *reinterpret_cast<const float4*>(ep.resid + (long)(mw + it * 4 + pr) * ep.ldo + n)
-                                : make_float4(0.f, 0.f, 0.f, 0.f);
-#pragma unroll
-              for (int it = 0; it < 8; ++it) {
-                if (ok[it]) {
-                  float4 o;
-                  o.x = t4[it].x + ep.alpha * a[it].x; o.y = t4[it].y + ep.alpha * a[it].y;
-                  o.z = t4[it].z + ep.alpha * a[it].z; o.w = t4[it].w + ep.alpha * a[it].w;
-                  *reinterpret_cast<float4*>(reinterpret_cast<float*>(ep.out) + (long)(mw + it * 4 + pr) * ep.ldo + n) = o;
-                }
-              }
-            }
-          }
-        }
-      }
-    }
     }  // tile loop
   }
   tc_fence_before();
@@ -509,58 +433,51 @@ static int num_sms() {
 }
 
 template <int MODE, int BN, int MSUB, typename TOp>
-static int launch_tc(const void* A, const void* Bw, int M, int N, int K, int splits, const EpiParams& ep,
-                     cudaStream_t st) {
+static int launch_tc(const void* A, const void* Bw, int M, int N, int K, const EpiParams& ep, cudaStream_t st) {
   using Cfg = TcCfg<BN, MSUB>;
   CUtensorMap tmA, tmB;
   AVSR_TRY(make_tmap_2d(&tmA, A, (uint64_t)M, (uint64_t)K, (uint64_t)K, TC_BM, (int)sizeof(TOp)));
   AVSR_TRY(make_tmap_2d(&tmB, Bw, (uint64_t)N, (uint64_t)K, (uint64_t)K, BN, (int)sizeof(TOp)));
   AVSR_SET_MAX_SMEM((gemm_tc_kernel<MODE, BN, MSUB, TOp>), Cfg::kSmem);
   const int tiles_m = cdiv(M, TC_BM * MSUB), tiles_n = cdiv(N, BN);
-  if (splits > kMaxSplits || tiles_m * tiles_n > kSplitCounters) splits = 1;   // caller's workspace contract
-  const int total = tiles_m * tiles_n * splits;
+  const int total = tiles_m * tiles_n;
   const int grid = total < num_sms() ? total : num_sms();
-  AVSR_LAUNCH((gemm_tc_kernel<MODE, BN, MSUB, TOp>), grid, TC_THREADS, Cfg::kSmem, st, tmA, tmB, K, tiles_m, tiles_n, splits, ep);
+  AVSR_LAUNCH((gemm_tc_kernel<MODE, BN, MSUB, TOp>), grid, TC_THREADS, Cfg::kSmem, st, tmA, tmB, K, tiles_m, tiles_n, ep);
   return AVSR_OK;
 }
 
-// ---------------------------------------------------------------- tile / split selection
+// ---------------------------------------------------------------- tile selection
 // Cost model (SM cycles) of one GEMM on 148 persistent CTAs.  What the r01 profiles showed: an SM ingests only
 // ~46 B/cycle through TMA (B300_MICROARCH "TMA service/SM"; measured 32 KB per ~690 cycles), well below what the
 // tensor pipe consumes, so time ~ (bytes pulled by the busiest SM) / 46 unless the tensor pipe is slower; the
-// epilogue hides behind the next item when the accumulator is double-buffered.  Split-K (only for GEMMs that
-// accumulate into the fp32 residual stream) spreads a long K over more SMs.
-struct TileChoice { int bn, msub, splits; };
+// epilogue hides behind the next tile when the accumulator is double-buffered.  (A deterministic split-K over the
+// residual-stream GEMMs was measured slower at S2, 2.45 vs 2.26 ms per forward: its fix-up re-reads the fp32
+// partial tiles through the same port as a serial tail.  It was removed; git history has it.)
+struct TileChoice { int bn, msub; };
 static const int kTileShapes[][2] = {{64, 1}, {128, 1}, {128, 2}, {256, 1}, {256, 2}};
 
-static TileChoice choose_tile(int mode, int M, int N, int K, int esz, bool operand_dest, bool can_split) {
+static TileChoice choose_tile(int mode, int M, int N, int K, int esz, bool operand_dest) {
   const double mac_per_cycle = esz == 2 ? 4096.0 : 2048.0;   // per SM, dense f16 / tf32
   const double ingest = 46.0;                                // TMA bytes per cycle per SM
   const int nkb = K / (128 / esz);
   const int sms = 148;
   double best = 1e30;
-  TileChoice pick{128, 1, 1};
+  TileChoice pick{128, 1};
   for (const auto& sh : kTileShapes) {
     const int bn = sh[0], msub = sh[1];
     if (mode == EPI_GLU && bn % 128 != 0) continue;
     if (bn == 64 && esz == 2 && (mode != EPI_LINEAR || operand_dest)) continue;   // needs 64-column row segments
     if (bn > 64 && N <= bn / 2) continue;                                          // mostly empty tile
     const long tiles = (long)cdiv(M, 128 * msub) * cdiv(N, bn);
-    for (int splits = 1; splits <= (can_split ? kMaxSplits : 1); ++splits) {
-      if (splits > nkb) break;
-      const long items = tiles * splits;
-      const long per_sm = (items + sms - 1) / sms;
-      const double kfrac = (double)((nkb + splits - 1) / splits) * (128 / esz);    // K elements of the longest slice
-      const double t_mma = per_sm * (double)msub * 128.0 * bn * kfrac / mac_per_cycle;
-      const double t_in = per_sm * ((double)msub * 128 + bn) * kfrac * esz / ingest;
-      const bool acc2 = 2 * msub * bn <= 512;
-      const double drain = (double)msub * bn * 10.0;                               // one item's epilogue
-      const double t_epi = acc2 ? drain : per_sm * drain;
-      // fix-up: the last arriver re-reads `splits` fp32 partial tiles through the same ~46 B/cycle port
-      const double t_red = splits > 1 ? (double)splits * msub * 128.0 * bn * 4.0 / ingest : 0.0;
-      const double est = (t_mma > t_in ? t_mma : t_in) + t_epi + t_red + 4000.0;
-      if (est < best) { best = est; pick = TileChoice{bn, msub, splits}; }
-    }
+    const long per_sm = (tiles + sms - 1) / sms;
+    const double kfrac = (double)nkb * (128 / esz);                               // K elements of a tile
+    const double t_mma = per_sm * (double)msub * 128.0 * bn * kfrac / mac_per_cycle;
+    const double t_in = per_sm * ((double)msub * 128 + bn) * kfrac * esz / ingest;
+    const bool acc2 = 2 * msub * bn <= 512;
+    const double drain = (double)msub * bn * 10.0;                                 // one tile's epilogue
+    const double t_epi = acc2 ? drain : per_sm * drain;
+    const double est = (t_mma > t_in ? t_mma : t_in) + t_epi + 4000.0;
+    if (est < best) { best = est; pick = TileChoice{bn, msub}; }
   }
   return pick;
 }
@@ -569,12 +486,12 @@ template <int MODE, typename TOp>
 static int dispatch_tile(TileChoice t, const void* A, const void* Bw, int M, int N, int K, const EpiParams& ep,
                          cudaStream_t st) {
   if (t.bn == 64) {
-    if constexpr (MODE != EPI_GLU) return launch_tc<MODE, 64, 1, TOp>(A, Bw, M, N, K, t.splits, ep, st);
+    if constexpr (MODE != EPI_GLU) return launch_tc<MODE, 64, 1, TOp>(A, Bw, M, N, K, ep, st);
   }
-  if (t.bn == 128 && t.msub == 1) return launch_tc<MODE, 128, 1, TOp>(A, Bw, M, N, K, t.splits, ep, st);
-  if (t.bn == 128 && t.msub == 2) return launch_tc<MODE, 128, 2, TOp>(A, Bw, M, N, K, t.splits, ep, st);
-  if (t.bn == 256 && t.msub == 1) return launch_tc<MODE, 256, 1, TOp>(A, Bw, M, N, K, t.splits, ep, st);
-  if (t.bn == 256 && t.msub == 2) return launch_tc<MODE, 256, 2, TOp>(A, Bw, M, N, K, t.splits, ep, st);
+  if (t.bn == 128 && t.msub == 1) return launch_tc<MODE, 128, 1, TOp>(A, Bw, M, N, K, ep, st);
+  if (t.bn == 128 && t.msub == 2) return launch_tc<MODE, 128, 2, TOp>(A, Bw, M, N, K, ep, st);
+  if (t.bn == 256 && t.msub == 1) return launch_tc<MODE, 256, 1, TOp>(A, Bw, M, N, K, ep, st);
+  if (t.bn == 256 && t.msub == 2) return launch_tc<MODE, 256, 2, TOp>(A, Bw, M, N, K, ep, st);
   set_error("gemm_tc: no kernel for tile %dx%d", t.msub * 128, t.bn);
   return AVSR_E_INVALID;
 }
@@ -583,25 +500,7 @@ template <typename TOp>
 static int dispatch_mode(int mode, const void* A, const void* Bw, int M, int N, int K, const EpiParams& ep,
                          cudaStream_t st) {
   const bool operand_dest = mode != EPI_GLU && (mode != EPI_LINEAR || ep.round_out != 0);
-  // split-K adds partial sums into the destination: only when the destination IS the residual it accumulates into
-  // Split-K needs the caller's fp32 workspace + zeroed tile counters (EpiParams::partial / counters); the slices
-  // are summed in fixed order by the last-arriving CTA, so the result does not depend on scheduling.  OPT-IN
-  // (AVSR_B200_SPLITK=1): measured at S2 it is SLOWER end to end (2.45 ms vs 2.26 ms per forward) -- the fix-up
-  // re-reads `splits` fp32 tiles through the same ~46 B/cycle/SM port the operands use, as a serial tail.  (The
-  // atomic variant, red.global.add.v4.f32, was 2.4 % faster but made the output vary run to run at the 2e-3 level.)
-  static const bool allow_split = [] { const char* e = getenv("AVSR_B200_SPLITK"); return e && e[0] == '1'; }();
-  const bool can_split = allow_split && mode == EPI_LINEAR && !ep.round_out && !ep.relu && ep.resid != nullptr &&
-                         ep.partial != nullptr && ep.counters != nullptr;
-  TileChoice t = choose_tile(mode, M, N, K, (int)sizeof(TOp), operand_dest, can_split);
-  if (const char* force = getenv("AVSR_B200_TILE")) {        // "BN,MSUB[,SPLITS]" -- tuning / profiling aid
-    int bn = 0, ms = 0, sp = 1;
-    const int got = sscanf(force, "%d,%d,%d", &bn, &ms, &sp);
-    if (got >= 2 && (mode != EPI_GLU || bn % 128 == 0) && !(bn == 64 && sizeof(TOp) == 2 && operand_dest)) {
-      if (got < 3 || !can_split || sp < 1) sp = 1;
-      const int nkb = K / (128 / (int)sizeof(TOp));
-      t = TileChoice{bn, ms, sp > nkb ? nkb : sp};
-    }
-  }
+  const TileChoice t = choose_tile(mode, M, N, K, (int)sizeof(TOp), operand_dest);
   AVSR_REQUIRE(mode == EPI_VT || N % 8 == 0, "gemm_tc: N=%d must be a multiple of 8", N);
   if (mode == EPI_LINEAR) {
     AVSR_REQUIRE((ep.ldo % 8) == 0 && (reinterpret_cast<uintptr_t>(ep.out) & 15) == 0 &&

@@ -131,9 +131,9 @@ struct T2Cfg {
 
 // RELU / RESID are compile-time: a predicated-off instruction still takes an issue slot, and this epilogue is not
 // overlapped with anything (one tile per cluster).
-// PREB (default inside the encoder forward, AVSR_B200_PREB=0 disables; prepared weights only; +0.6 % r02 A/B): the B operand (weights) does not depend on the
-// predecessor kernel, so the producer fills the B halves of the first stages BEFORE griddepcontrol.wait; after the
-// wait only the A tiles (just written by the predecessor, L2-resident) are still to come.
+// PREB (inside the encoder forward, whose B operands are prepared weights; +0.6 % in the r02 A/B): the B operand does
+// not depend on the predecessor kernel, so the producer fills the B halves of the first stages BEFORE
+// griddepcontrol.wait; after the wait only the A tiles (just written by the predecessor, L2-resident) are still to come.
 template <int MODE, int BNP, bool RELU, bool RESID, bool PREB = false>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(T2_THREADS, 1)
 gemm_tc2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB,
@@ -603,10 +603,6 @@ AVSR_TRACE_DEFINE_BIND(trace_bind_gemm_tc2)
 
 // set by encoder.cu around the forward schedule: B operands are prepared weights nobody writes during the forward
 thread_local bool g_tc2_weights_static = false;
-static bool preb_enabled() {
-  static const bool on = [] { const char* e = getenv("AVSR_B200_PREB"); return !(e && e[0] == '0'); }();
-  return on && g_tc2_weights_static && pdl_enabled();
-}
 
 template <int MODE, int BNP, bool RELU, bool RESID>
 static int launch_tc2_k(const CUtensorMap& tmA, const CUtensorMap& tmB, const CUtensorMap& tmB1, const CUtensorMap& tmOut,
@@ -615,7 +611,7 @@ static int launch_tc2_k(const CUtensorMap& tmA, const CUtensorMap& tmB, const CU
   using Cfg = T2Cfg<BNP, MODE, RESID>;
   AVSR_SET_MAX_SMEM((gemm_tc2_kernel<MODE, BNP, RELU, RESID>), Cfg::kSmem);
   const EpiParams& epl = ep;
-  if (preb_enabled()) {
+  if (g_tc2_weights_static) {
     AVSR_SET_MAX_SMEM((gemm_tc2_kernel<MODE, BNP, RELU, RESID, true>), Cfg::kSmem);
     AVSR_LAUNCH((gemm_tc2_kernel<MODE, BNP, RELU, RESID, true>), grid, T2_THREADS, Cfg::kSmem, st, tmA, tmB, tmB1, tmOut,
                 tmRes, K, tiles_n, nsplit, epl);
@@ -659,33 +655,25 @@ static int launch_tc2(const __half* A, const __half* Bw, int M, int N, int K, co
 // Deferred split-K plan for a residual GEMM whose consumer is a LayerNorm (the FFN w_2 projections, K = 3072):
 // with one 256 x 128 pair-tile per cluster only 84 SMs work and each ingests K * 384 * 2 bytes; slicing K over
 // `nsplit` clusters per (wider) pair-tile puts <= 74 clusters in one wave with 1/nsplit of the k-blocks each.
-// Returns 0 (no plan) or fills bnp / nsplit.  AVSR_B200_W2SPLIT = "0" | "<bnp>:<nsplit>" overrides.
-int gemm_tc2_splitk_plan(int M, int N, int K, int* bnp, int* nsplit) {
-  static const bool enabled = [] { const char* e = getenv("AVSR_B200_2CTA"); return !(e && e[0] == '0'); }();
-  if (!enabled || M < 256 || N % 8 != 0 || K % 64 != 0) return 0;
-  int wb = 256, ws = 3;
-  if (const char* e = getenv("AVSR_B200_W2SPLIT")) {
-    if (sscanf(e, "%d:%d", &wb, &ws) != 2) return 0;
-  }
-  if ((wb != 256 && wb != 384) || ws < 2 || ws > 4) return 0;   // LayerNorm consumers instantiated for 2, 3, 4 slices
-  const int tiles = cdiv(M, 256) * (N / wb);
-  if (N % wb != 0 || (K / 64) % ws != 0 || K / 64 / ws < 4 || tiles * ws > 74) return 0;
-  *bnp = wb; *nsplit = ws;
+// 256-wide pair-tiles x 3 slices beat 384 wide and 2 or 4 slices (profiles/r02_variants_ab.txt).
+// Returns 0 (no plan) or fills nsplit.
+constexpr int kSplitPairTile = 256;
+int gemm_tc2_splitk_plan(int M, int N, int K, int* nsplit) {
+  constexpr int ws = kW2Splits;   // the LayerNorm that consumes the slices is instantiated for this count
+  if (M < 256 || K % 64 != 0 || N % kSplitPairTile != 0) return 0;
+  const int tiles = cdiv(M, 256) * (N / kSplitPairTile);
+  if ((K / 64) % ws != 0 || K / 64 / ws < 4 || tiles * ws > 74) return 0;
+  *nsplit = ws;
   return 1;
 }
 
 // partial[s][M][N] (fp32, s < nsplit) = A[:, slice s of K] * Bw[:, slice s of K]^T -- no bias, no residual
-int gemm_tc2_splitk(const void* A, const void* Bw, int M, int N, int K, float* partial, int bnp, int nsplit,
-                    cudaStream_t st) {
+int gemm_tc2_splitk(const void* A, const void* Bw, int M, int N, int K, float* partial, int nsplit, cudaStream_t st) {
   EpiParams ep{};
   ep.M = M; ep.N = N; ep.out = partial; ep.ldo = N;
   AVSR_REQUIRE((reinterpret_cast<uintptr_t>(partial) & 15) == 0, "split-K partial buffer must be 16-byte aligned");
-  const __half* a = reinterpret_cast<const __half*>(A);
-  const __half* b = reinterpret_cast<const __half*>(Bw);
-  if (bnp == 384) return launch_tc2<EPI_LINEAR, 384>(a, b, M, N, K, ep, st, nsplit);
-  if (bnp == 256) return launch_tc2<EPI_LINEAR, 256>(a, b, M, N, K, ep, st, nsplit);
-  AVSR_REQUIRE(false, "split-K pair tile %d not instantiated", bnp);
-  return AVSR_OK;
+  return launch_tc2<EPI_LINEAR, kSplitPairTile>(reinterpret_cast<const __half*>(A), reinterpret_cast<const __half*>(Bw),
+                                                M, N, K, ep, st, nsplit);
 }
 
 int gemm_tc2_lse_ok(int M, int N, int K) { return M >= 256 && N % 512 == 0 && K % 64 == 0 && cdiv(M, 256) * (N / 512) <= 74; }
@@ -705,8 +693,7 @@ int gemm_tc2_lse(const void* A, const void* Bw, const float* bias, int M, int N,
 int gemm_tc2_try(int mode, const void* A, const void* Bw, int M, int N, int K, const EpiParams& ep, cudaStream_t st,
                  int* handled) {
   *handled = 0;
-  static const bool enabled = [] { const char* e = getenv("AVSR_B200_2CTA"); return !(e && e[0] == '0'); }();
-  if (!enabled || K % 64 != 0 || N % 8 != 0 || M < 256) return AVSR_OK;
+  if (K % 64 != 0 || N % 8 != 0 || M < 256) return AVSR_OK;
   if (mode != EPI_LINEAR && mode != EPI_QK && mode != EPI_GLU) return AVSR_OK;
   if (mode == EPI_LINEAR &&
       ((ep.ldo % 8) != 0 || (reinterpret_cast<uintptr_t>(ep.out) & 15) || (reinterpret_cast<uintptr_t>(ep.resid) & 15)))
