@@ -4,12 +4,12 @@ from __future__ import annotations
 
 import ctypes as C
 import os
-from collections import OrderedDict
 from typing import Dict, Optional, Tuple
 
 import torch
 
 from . import _cabi
+from ._cache import PlanCache, WorkspacePool, capture
 from ._cabi import EncoderConfig, LayerParams, LAYER_FIELDS, PREC_F16, PREC_FP32, PREC_TF32, check, lib
 
 PRECISIONS = {"fp32": PREC_FP32, "tf32": PREC_TF32, "f16": PREC_F16}
@@ -44,10 +44,10 @@ class EncoderEngine:
     """Runs ConformerEncoder.forward (eval) for one parameter set on one device.
 
     Shape policy (the reference's eval path feeds B=1 with a different T per utterance, lightning.py:72): a (B, T)
-    shape runs on direct launches -- one growable workspace per device, no capture cost -- until it has been seen
-    ``graph_after`` times; only then a CUDA-graph plan (own ~85 KB/frame workspace, ~190-node capture) is built for it.
-    Plans live in an LRU of ``MAX_PLANS`` (env AVSR_B200_MAX_PLANS).  Fixed-shape loops (training buckets, bench)
-    reach the graph after ``graph_after - 1`` calls; ``graph_after=1`` captures at first sight."""
+    shape runs on direct launches -- one grow-only workspace per (device, stream), no capture cost -- until it has been
+    seen ``graph_after`` times; only then a CUDA-graph plan (own ~85 KB/frame workspace, ~190-node capture) is built for
+    it.  ``plans`` keeps at most ``MAX_PLANS`` (env AVSR_B200_MAX_PLANS) in LRU order.  Fixed-shape loops (training
+    buckets, bench) reach the graph after ``graph_after - 1`` calls; ``graph_after=1`` captures at first sight."""
 
     MAX_PLANS = int(os.environ.get("AVSR_B200_MAX_PLANS", "16"))
     GRAPH_AFTER = int(os.environ.get("AVSR_B200_GRAPH_AFTER", "3"))
@@ -59,30 +59,24 @@ class EncoderEngine:
             check(_cabi.E_INVALID)
         self.prepared_bytes = need
         self._prepared: Dict[Tuple[int, int], torch.Tensor] = {}      # (device index, precision) -> buffer
-        self._workspaces: "OrderedDict[tuple, torch.Tensor]" = OrderedDict()
-        self._plans: "OrderedDict[tuple, tuple]" = OrderedDict()
-        self._seen: "OrderedDict[tuple, int]" = OrderedDict()        # shape key -> times seen (bounded)
-        self._capture_stream: Dict[int, torch.cuda.Stream] = {}
+        self._workspaces = WorkspacePool()
+        self.plans = PlanCache(lambda rec: lib.avsr_plan_destroy(rec[0]), self.GRAPH_AFTER, self.MAX_PLANS)
         self._sat: Dict[int, torch.Tensor] = {}
-        self.graph_after = self.GRAPH_AFTER
         self.stats = {"direct": 0, "graph": 0, "plans_built": 0}
+
+    @property
+    def graph_after(self) -> int:
+        return self.plans.graph_after
+
+    @graph_after.setter
+    def graph_after(self, n: int) -> None:
+        self.plans.graph_after = n
 
     # ---- weights -------------------------------------------------------------------------------
     def invalidate(self) -> None:
         """Forget prepared weights (and the plans that bake their addresses)."""
-        self._destroy_plans()
+        self.plans.clear()
         self._prepared.clear()
-
-    def _destroy_plans(self) -> None:
-        for plan, _ws in self._plans.values():
-            lib.avsr_plan_destroy(plan)
-        self._plans.clear()
-
-    def __del__(self):
-        try:
-            self._destroy_plans()
-        except Exception:
-            pass
 
     def prepare(self, state, device: torch.device, precision: str) -> torch.Tensor:
         """state: reference-keyed tensors ('encoders.{l}.<suffix>', 'after_norm.*') living on `device`, or a
@@ -115,18 +109,6 @@ class EncoderEngine:
         self._prepared[key] = buf
         return buf
 
-    # ---- buffers -------------------------------------------------------------------------------
-    def _workspace(self, B: int, T: int, device: torch.device, stream: int) -> torch.Tensor:
-        """The direct-launch workspace: ONE buffer per (device, stream), grown to the largest shape seen (its layout
-        is carved per call by the library, so any buffer that is large enough serves every shape)."""
-        key = (device.index or 0, stream)
-        nbytes = max(int(lib.avsr_workspace_bytes(C.byref(self.cfg), B, T)), 256)
-        ws = self._workspaces.get(key)
-        if ws is None or ws.numel() < nbytes:
-            ws = torch.empty(nbytes + nbytes // 4, dtype=torch.uint8, device=device)   # 25 % slack: fewer regrowths
-            self._workspaces[key] = ws
-        return ws
-
     # ---- forward -------------------------------------------------------------------------------
     def forward(self, prepared: torch.Tensor, xs: torch.Tensor, lengths: Optional[torch.Tensor], precision: str,
                 use_graph: bool = True, taps: Optional[torch.Tensor] = None, check_saturation: bool = False) -> torch.Tensor:
@@ -146,15 +128,16 @@ class EncoderEngine:
         prec = PRECISIONS[precision]
         with torch.cuda.device(device):
             st = _stream_handle(device)
-            plan = None
+            rec = None
             if use_graph and taps is None and not check_saturation:
-                plan = self._plan(prepared, B, T, device, prec, st)
-            if plan is not None:
+                rec = self.plans.get((device.index or 0, B, T, prec, prepared.data_ptr(), st),
+                                     lambda: self._build_plan(prepared, B, T, device, prec))
+            if rec is not None:
                 self.stats["graph"] += 1
-                check(lib.avsr_plan_forward(plan, xs.data_ptr(), _ptr(lengths), out.data_ptr(), st))
+                check(lib.avsr_plan_forward(rec[0], xs.data_ptr(), _ptr(lengths), out.data_ptr(), st))
             else:
                 self.stats["direct"] += 1
-                ws = self._workspace(B, T, device, st)
+                ws = self._workspaces.get("direct", int(lib.avsr_workspace_bytes(C.byref(self.cfg), B, T)), device, st)
                 if check_saturation:
                     cnt = self._sat.get(device.index or 0)
                     if cnt is None:
@@ -176,34 +159,11 @@ class EncoderEngine:
                                                         ws.data_ptr(), ws.numel(), prec, st))
         return out
 
-    def _plan(self, prepared: torch.Tensor, B: int, T: int, device: torch.device, prec: int, stream: int):
-        """The plan for this shape, or None while the shape has been seen fewer than ``graph_after`` times.  A plan's
-        workspace is private to it and to the stream it was built for (two streams never share one)."""
-        key = (device.index or 0, B, T, prec, prepared.data_ptr(), stream)
-        hit = self._plans.get(key)
-        if hit is not None:
-            self._plans.move_to_end(key)
-            return hit[0]
-        seen = self._seen.get(key, 0) + 1
-        self._seen[key] = seen
-        self._seen.move_to_end(key)
-        while len(self._seen) > 64 * self.MAX_PLANS:
-            self._seen.popitem(last=False)
-        if seen < self.graph_after:
-            return None
+    def _build_plan(self, prepared: torch.Tensor, B: int, T: int, device: torch.device, prec: int) -> tuple:
+        """(plan, its workspace) for one shape.  The workspace is private to the plan, so to the stream in its key."""
         self.stats["plans_built"] += 1
         ws = torch.empty(int(lib.avsr_workspace_bytes(C.byref(self.cfg), B, T)), dtype=torch.uint8, device=device)
-        idx = device.index or 0
-        if idx not in self._capture_stream:
-            self._capture_stream[idx] = torch.cuda.Stream(device=device)   # the legacy default stream cannot capture
-        cs = self._capture_stream[idx]
-        cs.wait_stream(torch.cuda.current_stream(device))
         plan = C.c_void_p()
-        check(lib.avsr_plan_create(C.byref(self.cfg), prepared.data_ptr(), B, T, ws.data_ptr(), ws.numel(), prec,
-                                   cs.cuda_stream, C.byref(plan)))
-        cs.synchronize()
-        self._plans[key] = (plan, ws)
-        while len(self._plans) > self.MAX_PLANS:
-            _, (old, _ws) = self._plans.popitem(last=False)
-            lib.avsr_plan_destroy(old)
-        return plan
+        capture(device, lambda cs: check(lib.avsr_plan_create(C.byref(self.cfg), prepared.data_ptr(), B, T, ws.data_ptr(),
+                                                               ws.numel(), prec, cs, C.byref(plan))))
+        return plan, ws

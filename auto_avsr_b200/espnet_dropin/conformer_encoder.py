@@ -203,7 +203,14 @@ class ConformerEncoder(torch.nn.Module):
         self._tracked = None
         self._fingerprint = None
         if getattr(self, "_engine", None) is not None:
-            self._engine.invalidate()
+            self._invalidate()
+
+    def _invalidate(self) -> None:
+        """Forget the prepared weights and every plan that bakes their address: the engine's and the fused head's."""
+        self._engine.invalidate()
+        head = getattr(self, "_fused_head", None)
+        if head is not None:
+            head.plans.clear()
 
     def _weights_fingerprint(self):
         if self._tracked is None:
@@ -219,7 +226,7 @@ class ConformerEncoder(torch.nn.Module):
         if not (self.assume_frozen and self._fingerprint is not None):
             fp = self._weights_fingerprint()
             if fp != self._fingerprint:
-                self._engine.invalidate()
+                self._invalidate()
                 self._fingerprint = fp
         return self._engine.prepare(lambda: self.state_dict(keep_vars=True), device, precision)
 

@@ -13,29 +13,17 @@ from typing import Dict, Optional, Tuple
 import torch
 
 from ._cabi import EncoderConfig, check, lib
-from .engine import PRECISIONS, _ptr, _stream_handle, default_precision, require_cuda
+from ._cache import PlanCache, WorkspacePool, capture
+from .engine import PRECISIONS, EncoderEngine, _ptr, _stream_handle, default_precision, require_cuda
 
 
 class PreparedHead:
     def __init__(self, d_model: int, n_heads: int = 12, linear_units: int = 3072, num_blocks: int = 12, cnn_kernel: int = 31):
         self.cfg = EncoderConfig(d_model, n_heads, linear_units, num_blocks, cnn_kernel)
         self._buf: Dict[tuple, Tuple[tuple, torch.Tensor]] = {}
-        self._ws: Dict[tuple, torch.Tensor] = {}
-        self._plans: Dict[tuple, tuple] = {}          # shape key -> (plan, workspace, enc_out, logp, argmax)
-        self._seen: Dict[tuple, int] = {}
-        self._capture_stream: Dict[int, torch.cuda.Stream] = {}
-
-    def __del__(self):
-        try:
-            for plan, *_ in self._plans.values():
-                lib.avsr_plan_destroy(plan)
-        except Exception:
-            pass
-
-    def drop_plans(self) -> None:
-        for plan, *_ in self._plans.values():
-            lib.avsr_plan_destroy(plan)
-        self._plans.clear()
+        self.workspaces = WorkspacePool()
+        # plans of features_to_log_probs: (plan, workspace, enc_out, logp, argmax)
+        self.plans = PlanCache(lambda rec: lib.avsr_plan_destroy(rec[0]), EncoderEngine.GRAPH_AFTER, EncoderEngine.MAX_PLANS)
 
     @staticmethod
     def _fp(*tensors) -> tuple:
@@ -65,16 +53,8 @@ class PreparedHead:
             check(lib.avsr_prepare_head(C.byref(self.cfg), idim, odim, _ptr(pw), _ptr(pb), _ptr(cw), _ptr(cb),
                                         buf.data_ptr(), nbytes, PRECISIONS[precision], _stream_handle(device)))
         self._buf[key] = (fp, buf)
-        self.drop_plans()                       # plans bake the prepared buffers' addresses
+        self.plans.clear()                      # plans bake the prepared buffers' addresses
         return buf, idim, odim
-
-    def workspace(self, tag: str, nbytes: int, device) -> torch.Tensor:
-        key = (tag, device.index or 0, _stream_handle(device))
-        ws = self._ws.get(key)
-        if ws is None or ws.numel() < nbytes:
-            ws = torch.empty(max(nbytes + nbytes // 4, 256), dtype=torch.uint8, device=device)
-            self._ws[key] = ws
-        return ws
 
 
 def proj_forward(head: PreparedHead, proj: torch.nn.Linear, x: torch.Tensor, precision: str) -> torch.Tensor:
@@ -84,7 +64,7 @@ def proj_forward(head: PreparedHead, proj: torch.nn.Linear, x: torch.Tensor, pre
     buf, idim, odim = head.prepare(proj, None, x.device, precision)
     rows = x.numel() // idim
     y = torch.empty(*x.shape[:-1], head.cfg.d_model, dtype=torch.float32, device=x.device)
-    ws = head.workspace("proj", rows * idim * 4 + 256, x.device)
+    ws = head.workspaces.get("proj", rows * idim * 4 + 256, x.device, _stream_handle(x.device))
     with torch.cuda.device(x.device):
         check(lib.avsr_proj_encoder(C.byref(head.cfg), buf.data_ptr(), x.data_ptr(), rows, idim, odim, y.data_ptr(),
                                     ws.data_ptr(), ws.numel(), PRECISIONS[precision], _stream_handle(x.device)))
@@ -101,7 +81,7 @@ def ctc_log_probs(head: PreparedHead, ctc_lo: torch.nn.Linear, hs: torch.Tensor,
     logp = torch.empty(*hs.shape[:-1], odim, dtype=torch.float32, device=hs.device) if want_logp else None
     best = torch.empty(hs.shape[:-1], dtype=torch.int32, device=hs.device) if want_argmax else None
     nbytes = int(lib.avsr_ctc_workspace_bytes(C.byref(head.cfg), rows, odim))
-    ws = head.workspace("ctc", nbytes, hs.device)
+    ws = head.workspaces.get("ctc", nbytes, hs.device, _stream_handle(hs.device))
     with torch.cuda.device(hs.device):
         check(lib.avsr_ctc_logprobs(C.byref(head.cfg), buf.data_ptr(), hs.data_ptr(), rows, idim, odim, _ptr(logp),
                                     _ptr(best), ws.data_ptr(), ws.numel(), PRECISIONS[precision], _stream_handle(hs.device)))
@@ -135,38 +115,26 @@ def features_to_log_probs(proj: torch.nn.Linear, encoder, ctc, feats: torch.Tens
     if head is None:
         head = encoder._fused_head = PreparedHead(*encoder._cfg)
     hbuf, idim, odim = head.prepare(proj, ctc.ctc_lo, dev, precision)
+    st = _stream_handle(dev)
     if B and T and encoder.use_graph and not getattr(encoder, "check_saturation", False):
-        # CUDA-graph replay once the shape has been seen `graph_after` times (same policy as the encoder's own plans).
-        # The plan owns its output tensors: the ones returned here are overwritten by the next call with this shape.
-        st = _stream_handle(dev)
-        key = (dev.index or 0, B, T, idim, odim, PRECISIONS[precision], prepared.data_ptr(), hbuf.data_ptr(), st,
-               want_features, want_argmax)
-        hit = head._plans.get(key)
-        if hit is None:
-            seen = head._seen[key] = head._seen.get(key, 0) + 1
-            if seen >= encoder._engine.graph_after:
-                nbytes = int(lib.avsr_head_plan_workspace_bytes(C.byref(head.cfg), B, T, idim, odim))
-                ws = torch.empty(nbytes, dtype=torch.uint8, device=dev)
-                eo = torch.empty(B, T, head.cfg.d_model, dtype=torch.float32, device=dev) if want_features else None
-                lp = torch.empty(B, T, odim, dtype=torch.float32, device=dev)
-                am = torch.empty(B, T, dtype=torch.int32, device=dev) if want_argmax else None
-                idx = dev.index or 0
-                if idx not in head._capture_stream:
-                    head._capture_stream[idx] = torch.cuda.Stream(device=dev)
-                cs = head._capture_stream[idx]
-                cs.wait_stream(torch.cuda.current_stream(dev))
-                plan = C.c_void_p()
-                with torch.cuda.device(dev):
-                    check(lib.avsr_head_plan_create(C.byref(head.cfg), prepared.data_ptr(), hbuf.data_ptr(), B, T, idim, odim,
-                                                    _ptr(eo), lp.data_ptr(), _ptr(am), ws.data_ptr(), nbytes,
-                                                    PRECISIONS[precision], cs.cuda_stream, C.byref(plan)))
-                cs.synchronize()
-                hit = head._plans[key] = (plan, ws, eo, lp, am)
-                while len(head._plans) > encoder._engine.MAX_PLANS:
-                    old = head._plans.pop(next(iter(head._plans)))
-                    lib.avsr_plan_destroy(old[0])
-        if hit is not None:
-            plan, _ws, eo, lp, am = hit
+        # CUDA-graph replay under the encoder's shape policy and threshold.  The plan owns its output tensors: the ones
+        # returned here are overwritten by the next call with this shape.
+        def build():
+            nbytes = int(lib.avsr_head_plan_workspace_bytes(C.byref(head.cfg), B, T, idim, odim))
+            ws = torch.empty(nbytes, dtype=torch.uint8, device=dev)
+            eo = torch.empty(B, T, head.cfg.d_model, dtype=torch.float32, device=dev) if want_features else None
+            lp = torch.empty(B, T, odim, dtype=torch.float32, device=dev)
+            am = torch.empty(B, T, dtype=torch.int32, device=dev) if want_argmax else None
+            plan = C.c_void_p()
+            capture(dev, lambda cs: check(lib.avsr_head_plan_create(
+                C.byref(head.cfg), prepared.data_ptr(), hbuf.data_ptr(), B, T, idim, odim, _ptr(eo), lp.data_ptr(),
+                _ptr(am), ws.data_ptr(), nbytes, PRECISIONS[precision], cs, C.byref(plan))))
+            return plan, ws, eo, lp, am
+        head.plans.graph_after = encoder._engine.graph_after
+        rec = head.plans.get((dev.index or 0, B, T, idim, odim, PRECISIONS[precision], prepared.data_ptr(),
+                              hbuf.data_ptr(), st, want_features, want_argmax), build)
+        if rec is not None:
+            plan, _ws, eo, lp, am = rec
             with torch.cuda.device(dev):
                 check(lib.avsr_head_plan_forward(plan, feats.data_ptr(), _ptr(lengths), st))
             return eo, lp, (None if am is None else am.long())
@@ -175,10 +143,9 @@ def features_to_log_probs(proj: torch.nn.Linear, encoder, ctc, feats: torch.Tens
     best = torch.empty(B, T, dtype=torch.int32, device=dev) if want_argmax else None
     if B and T:
         nbytes = int(lib.avsr_head_workspace_bytes(C.byref(head.cfg), B, T, idim, odim))
-        ws = head.workspace("fused", nbytes, dev)
+        ws = head.workspaces.get("fused", nbytes, dev, st)
         with torch.cuda.device(dev):
             check(lib.avsr_features_to_logprobs(C.byref(head.cfg), prepared.data_ptr(), hbuf.data_ptr(), feats.data_ptr(),
                                                 _ptr(lengths), B, T, idim, odim, _ptr(enc_out), logp.data_ptr(),
-                                                _ptr(best), ws.data_ptr(), ws.numel(), PRECISIONS[precision],
-                                                _stream_handle(dev)))
+                                                _ptr(best), ws.data_ptr(), ws.numel(), PRECISIONS[precision], st))
     return enc_out, logp, (None if best is None else best.long())

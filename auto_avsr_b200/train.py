@@ -20,17 +20,10 @@ import torch
 
 from . import ops
 from ._cabi import check, lib
+from ._cache import WorkspacePool
 from .engine import _ptr, _stream_handle, require_cuda
 
-_WS = {}
-
-
-def _workspace(device, nbytes: int) -> torch.Tensor:
-    key = (device.index or 0, _stream_handle(device))
-    ws = _WS.get(key)
-    if ws is None or ws.numel() < nbytes:
-        ws = _WS[key] = torch.empty(nbytes + nbytes // 4 + 1024, dtype=torch.uint8, device=device)
-    return ws
+_pool = WorkspacePool()
 
 
 def _c(t: torch.Tensor) -> torch.Tensor:
@@ -47,7 +40,7 @@ def layernorm_bwd(x, gamma, dy):
     d = x.size(-1)
     rows = x.numel() // d
     dx, dg, db = torch.empty_like(x), torch.empty_like(gamma), torch.empty_like(gamma)
-    ws = _workspace(x.device, int(lib.avsr_train_workspace_bytes(rows, d, 1)))
+    ws = _pool.get("train", int(lib.avsr_train_workspace_bytes(rows, d, 1)), x.device, _stream_handle(x.device))
     with torch.cuda.device(x.device):
         check(lib.avsr_layernorm_bwd(x.data_ptr(), gamma.data_ptr(), dy.data_ptr(), dx.data_ptr(), dg.data_ptr(), db.data_ptr(),
                                      rows, d, ws.data_ptr(), ws.numel(), _stream_handle(x.device)))
@@ -59,7 +52,7 @@ def colsum(y):
     cols = y.size(-1)
     rows = y.numel() // cols
     out = torch.empty(cols, dtype=torch.float32, device=y.device)
-    ws = _workspace(y.device, 148 * cols * 4 + 1024)
+    ws = _pool.get("train", 148 * cols * 4 + 1024, y.device, _stream_handle(y.device))
     with torch.cuda.device(y.device):
         check(lib.avsr_colsum(y.data_ptr(), out.data_ptr(), rows, cols, ws.data_ptr(), ws.numel(), _stream_handle(y.device)))
     return out
@@ -175,7 +168,7 @@ def _chan_sums(v, dy=None, mean=None, invstd=None, gamma=None, beta=None):
     Cc = v.size(-1)
     rows = v.numel() // Cc
     out = torch.empty(2, Cc, dtype=torch.float32, device=v.device)
-    ws = _workspace(v.device, 148 * 2 * Cc * 4 + 1024)
+    ws = _pool.get("train", 148 * 2 * Cc * 4 + 1024, v.device, _stream_handle(v.device))
     with torch.cuda.device(v.device):
         check(lib.avsr_chan_sums(v.data_ptr(), _ptr(dy), _ptr(mean), _ptr(invstd), _ptr(gamma), _ptr(beta), out.data_ptr(),
                                  rows, Cc, ws.data_ptr(), ws.numel(), _stream_handle(v.device)))
@@ -186,7 +179,7 @@ def _dwconv_raw(x, w, b, flip: bool):
     B, T, Cc = x.shape
     K = w.size(-1)
     y = torch.empty_like(x)
-    ws = _workspace(x.device, (K + 2) * Cc * 4 + 1024)
+    ws = _pool.get("train", (K + 2) * Cc * 4 + 1024, x.device, _stream_handle(x.device))
     with torch.cuda.device(x.device):
         check(lib.avsr_dwconv_raw(x.data_ptr(), w.data_ptr(), _ptr(b), y.data_ptr(), B, T, Cc, K, int(flip), ws.data_ptr(),
                                   ws.numel(), _stream_handle(x.device)))
@@ -251,7 +244,7 @@ class DwConvBnSiluFn(torch.autograd.Function):
                                           float(ctx.inv_count), dconv.data_ptr(), B * T, Cc, _stream_handle(x.device)))
         dx = _dwconv_raw(dconv, w, None, True)                             # correlation with the flipped taps
         dw, db = torch.empty_like(w), torch.empty(Cc, device=x.device)
-        ws = _workspace(x.device, int(lib.avsr_train_workspace_bytes(B * T, Cc, K)))
+        ws = _pool.get("train", int(lib.avsr_train_workspace_bytes(B * T, Cc, K)), x.device, _stream_handle(x.device))
         with torch.cuda.device(x.device):
             check(lib.avsr_dwconv_wgrad(x.data_ptr(), dconv.data_ptr(), dw.data_ptr(), db.data_ptr(), B, T, Cc, K, ws.data_ptr(),
                                         ws.numel(), _stream_handle(x.device)))
@@ -280,7 +273,7 @@ class AttentionCoreFn(torch.autograd.Function):
         dq_k, dq_p, dk, dv = (torch.empty_like(q) for _ in range(4))
         dp = torch.empty_like(p)
         ln = lengths.to(torch.int32).contiguous() if ctx_.masked else None
-        ws = _workspace(q.device, int(lib.avsr_relpos_attention_bwd_workspace_bytes(B, T, H)))
+        ws = _pool.get("train", int(lib.avsr_relpos_attention_bwd_workspace_bytes(B, T, H)), q.device, _stream_handle(q.device))
         with torch.cuda.device(q.device):
             check(lib.avsr_relpos_attention_bwd(q.data_ptr(), k.data_ptr(), v.data_ptr(), p.data_ptr(), u.data_ptr(),
                                                 vb.data_ptr(), _ptr(ln), out.data_ptr(), dctx.data_ptr(), dq_k.data_ptr(),

@@ -153,6 +153,9 @@ assert torch.logsumexp(logp.double().cpu(), -1).abs().max() < 1e-4
 assert torch.equal(best.cpu(), logp.argmax(-1).cpu())
 agree = (best.cpu() == torch.from_numpy(z["argmax_f64"])).float().mean().item()
 assert agree >= (0.99 if {prec!r} == "fp32" else 0.9), agree
+assert len(enc._fused_head.plans) == 2                # one per (want_features, want_argmax) combination used above
+enc.refresh_weights()                                 # the encoder's prepared weights go, and the fused plans baking them
+assert len(enc._fused_head.plans) == 0
 print("CHILD-OK")
 """)
 
